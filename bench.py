@@ -1,6 +1,6 @@
 """Benchmark of the UNet-ConvLSTM training step (BASELINE.json metric: train sequences/s, fwd+bwd).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): Moving-MNIST-shaped sequences 64x64, T=20, batch 256 per GPU,
@@ -13,8 +13,10 @@ Prints ONE JSON line (rank 0).  `value`: inputs resident in HBM.  `e2e`: same st
 nn.Module API with the batch in pinned host memory (H2D inside the timed region, loss read back).
 `roofline`: the fused ConvLSTM gate-conv kernel, timed per launch with CUDA events inside the timed
 region.  `cpu_baseline` / `--impl reference`: the UNMODIFIED reference (its train/unet.py model and main.py
-compute_loss, from /root/reference or the git-ignored copy baseline/_ref that travels to the GPU box; kind
-"reference") on this box's host cores, on a bounded sample; oracle/torch_port.py (kind "port") only if no copy exists.
+compute_loss, from the checkout B200_REFERENCE_DIR names; kind "reference") on this box's host cores, on a bounded
+sample; oracle/torch_port.py (kind "port") when no checkout is named.
+`--dump-outputs DIR`: after the timed steps, what the last of them computed is written to DIR as float32 .npy files
+(see dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -24,6 +26,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -83,19 +86,19 @@ def loss_torch(y_pred, y, mask):
 
 
 # ------------------------------------------------------------------------------------------------
-def clocks_sampler_start(gpu_index, path):
+def clocks_sampler_start(gpu_index):
     q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
          "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
          "clocks_event_reasons.sw_power_cap")
     try:
-        f = open(path, "w")
+        f = tempfile.TemporaryFile("w+")  # not in the tree: bench.py writes nothing there
         return subprocess.Popen(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-lms", "200",
                                  "-i", str(gpu_index)], stdout=f, stderr=subprocess.DEVNULL), f
     except OSError:
         return None, None
 
 
-def clocks_summary(proc, f, path):
+def clocks_summary(proc, f):
     if proc is None:
         return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
     proc.terminate()
@@ -103,10 +106,12 @@ def clocks_summary(proc, f, path):
         proc.wait(timeout=5)
     except subprocess.TimeoutExpired:
         proc.kill()
+    f.seek(0)
+    lines = f.readlines()
     f.close()
     sm, smax, reasons = [], None, set()
     names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
-    for line in open(path):
+    for line in lines:
         c = [v.strip() for v in line.split(",")]
         if len(c) < 9:
             continue
@@ -141,10 +146,9 @@ def host_info():
 # the reference's CPU path (oracle/torch_port.py) -- cpu_baseline leg and --impl reference
 # ------------------------------------------------------------------------------------------------
 def load_reference():
-    """The UNMODIFIED reference (train/unet.py's TemporalUNetDualView, main.py's compute_loss) from /root/reference or
-    its git-ignored copy baseline/_ref (made by __graft_entry__.build(); it travels to the GPU box).  Loaded by file
-    path under private module names, so this repository's own `train.unet` stays what `import train.unet` means.
-    Returns (model class, compute_loss, source dir) or None when neither directory exists."""
+    """The UNMODIFIED reference (train/unet.py's TemporalUNetDualView, main.py's compute_loss) from the checkout
+    B200_REFERENCE_DIR names.  Loaded by file path under private module names, so this repository's own `train.unet`
+    stays what `import train.unet` means.  Returns (model class, compute_loss, source dir) or None without a checkout."""
     import importlib.util
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     try:
@@ -295,13 +299,17 @@ def run_b200_arm(args, out):
     x_host, y_host, m_host = x_host.pin_memory(), y_host.pin_memory(), m_host.pin_memory()
     x_dev, y_dev, m_dev = x_host.to(dev), y_host.to(dev), m_host.to(dev)
     params = [q for q in model.parameters() if q.requires_grad]
+    last = {}  # with --dump-outputs: the predictions and loss of the last timed step
 
-    def step(x, y, m, with_opt=True):
+    def step(x, y, m, with_opt=True, keep=False):
         # the reference's training step (main.py:94-108): forward, compute_loss, backward, clip_grad_norm_(1.0),
         # optimizer step
         opt.zero_grad(set_to_none=True)
         out, _ = model(x)
-        loss = compute_loss(torch.stack(out, dim=1), y, m)
+        y_pred = torch.stack(out, dim=1)
+        loss = compute_loss(y_pred, y, m)
+        if keep:
+            last.update(pred=y_pred.detach(), loss=loss.detach())
         loss.backward()
         if reducer is not None:
             reducer.finish()
@@ -403,17 +411,24 @@ def run_b200_arm(args, out):
                 rate = f"{d[3] / d[1] / 1e6:8.1f} GB/s"
             print(f"# {d[1]:9.3f} ms {100 * d[1] / tot:5.1f}% x{d[0]:<4d} {rate:>18s}  {label}", file=sys.stderr)
 
-    clk_path = os.path.join(ROOT, "gpurun_out", f"bench_clocks_r{rank}.csv")
-    os.makedirs(os.path.dirname(clk_path), exist_ok=True)
-    proc, f = clocks_sampler_start(local, clk_path) if rank == 0 else (None, None)
+    proc, f = clocks_sampler_start(local) if rank == 0 else (None, None)
 
     # ---- eager region: every launch from Python, CUDA events around each fused cell launch (roofline) ----
     ops.CELL_TIMER = []
     calls0 = _lib.kernel_launches()
-    ms_eager = timed(lambda: step(x_dev, y_dev, m_dev), args.steps, tag="value")
+    steps_done = [0]
+
+    def value_step():
+        steps_done[0] += 1
+        return step(x_dev, y_dev, m_dev, keep=bool(args.dump_outputs) and rank == 0 and steps_done[0] == args.steps)
+
+    ms_eager = timed(value_step, args.steps, tag="value")
     launches = _lib.kernel_launches() - calls0
     cell_events, ops.CELL_TIMER = ops.CELL_TIMER, None
     torch.cuda.synchronize()
+    if last:
+        dump_outputs(args.dump_outputs, last, model)
+        last.clear()
     cell_ms = [a.elapsed_time(b) for a, b, _ in cell_events]
     cell_flops = [fl for _, _, fl in cell_events]
 
@@ -442,7 +457,7 @@ def run_b200_arm(args, out):
     e2e_region(2)
     ms_e2e = timed(lambda: e2e_region(args.steps), 1) / args.steps
 
-    clocks = clocks_summary(proc, f, clk_path) if rank == 0 else None
+    clocks = clocks_summary(proc, f) if rank == 0 else None
     peak_mem = torch.cuda.max_memory_allocated(dev)
 
     if rank == 0:
@@ -501,6 +516,37 @@ def run_b200_arm(args, out):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64_000_000
+DUMP_PARAM_SAMPLE = 4096
+NPY_HEADER = 256  # upper bound of the header np.save writes in front of the data
+
+
+def dump_outputs(path, last, model):
+    """Writes what the last timed step computed to `path`, float32: loss.npy (the scalar loss), pred.npy (the predictions
+    [B', T, 1, H, W] of B' of the B sequences, a seeded choice so the files stay under DUMP_BYTES) and
+    param.<name>.npy (each parameter after the optimizer step, or a seeded sample of DUMP_PARAM_SAMPLE of its elements
+    in flat order)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0)
+    arrays = {"loss": last["loss"].detach().float().reshape(())}
+    for name, p in model.named_parameters():
+        flat = p.detach().float().reshape(-1)
+        if flat.numel() > DUMP_PARAM_SAMPLE:
+            idx = np.sort(rng.choice(flat.numel(), DUMP_PARAM_SAMPLE, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        arrays[f"param.{name}"] = flat
+    pred = last["pred"].detach().float()
+    room = DUMP_BYTES - sum(a.numel() * 4 + NPY_HEADER for a in arrays.values()) - NPY_HEADER
+    keep = min(pred.shape[0], room // (pred[0].numel() * 4))
+    if keep < pred.shape[0]:
+        idx = np.sort(rng.choice(pred.shape[0], keep, replace=False))
+        pred = pred[torch.from_numpy(idx).to(pred.device)]
+    arrays["pred"] = pred
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
+
+
 def _claim_stdout():
     """The contract is ONE JSON line on stdout: libraries that print there (NCCL's version banner on
     rank 0) are sent to stderr; the JSON line goes to the saved descriptor."""
@@ -526,7 +572,13 @@ def main():
     ap.add_argument("--breakdown", action="store_true", help="print a per-entry-point time table to stderr")
     ap.add_argument("--timeline", default="", help="with --breakdown: write start/end/stream of every C-ABI call to this CSV")
     ap.add_argument("--profile-steps", type=int, default=0, help="run 1 warm-up + N untimed steps and exit (for ncu)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the loss, predictions and updated parameters of the last timed step to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path computed: not with --impl reference")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     out = _claim_stdout()

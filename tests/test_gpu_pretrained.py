@@ -8,7 +8,8 @@ strides 1, 2, 4, 8, 16, 32, decoder(*features), segmentation_head) built from st
 third-party code in the reference as well and stay on stock PyTorch.  What is compared is the same model object graph
 with the ConvLSTMs of this repository against the ConvLSTMs of the reference (same weights, same input): output and
 the gradients of every trainable parameter.  The 2-channel full-resolution cell runs on the CUDA-core path, the others
-on tcgen05."""
+on tcgen05.  train/resnet18.py is the reference project's, which this repository does not ship: the test runs when
+B200_REFERENCE_DIR names a checkout of it and is skipped otherwise."""
 import os
 import sys
 import types
@@ -18,9 +19,16 @@ import pytest
 import torch
 import torch.nn as nn
 
-pytestmark = pytest.mark.gpu
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+try:
+    import run_reference as RR
+finally:
+    sys.path.pop(0)
+REF = RR.find_reference()
+
+pytestmark = [pytest.mark.gpu,
+              pytest.mark.skipif(REF is None, reason="needs the reference project's train/resnet18.py: set B200_REFERENCE_DIR")]
 CH = (2, 64, 64, 128, 256, 512)
 
 
@@ -61,18 +69,13 @@ class _Unet(nn.Module):
 
 
 def _load(impl):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    try:
-        import run_reference as RR
-    finally:
-        sys.path.pop(0)
     RR.set_paths(impl)
     smp = types.ModuleType("segmentation_models_pytorch")
     smp.Unet = _Unet
     sys.modules["segmentation_models_pytorch"] = smp
     import importlib
     mod = importlib.import_module("train.resnet18")
-    assert os.path.basename(os.path.dirname(os.path.dirname(mod.__file__))) in ("reference", "_ref")
+    assert os.path.dirname(os.path.dirname(mod.__file__)) == REF
     return mod
 
 
@@ -118,6 +121,5 @@ def test_pretrained_temporal_unet_on_b200_convlstm():
         sys.modules.pop("segmentation_models_pytorch", None)
         for k in [k for k in sys.modules if k == "train" or k.startswith("train.")]:
             del sys.modules[k]
-        for p in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-            while p in sys.path:
-                sys.path.remove(p)
+        while REF in sys.path:
+            sys.path.remove(REF)

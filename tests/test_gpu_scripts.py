@@ -1,8 +1,9 @@
 """The reference's scripts, UNCHANGED, on top of this repository's train/unet.py (VERDICT r01 item 4, north_star "so
 main.py, train/overfit_check.py and train/get_metrics.py run unchanged ... the overfit_check loss curve matches within
-tolerance").  tools/run_reference.py executes the scripts from their own source files (baseline/_ref on the GPU box)
-and only supplies environment: import path order, stubs for the absent smp / matplotlib, the torch-2.11 keyword
-shims, constant overrides, a synthetic NPZ.
+tolerance").  tools/run_reference.py executes the scripts from their own source files and only supplies environment:
+import path order, stubs for the absent smp / matplotlib, the torch-2.11 keyword shims, constant overrides, a synthetic
+NPZ.  The scripts are the reference project's, which this repository does not ship: these tests run when
+B200_REFERENCE_DIR names a checkout of it and are skipped otherwise.
 
 The A/B partner (--impl reference) is the reference's own train/unet.py through stock PyTorch on the same GPU
 (cuDNN, TF32 off): same script, same seeds, same NPZ.
@@ -14,10 +15,17 @@ import sys
 
 import pytest
 
-pytestmark = pytest.mark.gpu
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TOOL = os.path.join(ROOT, "tools", "run_reference.py")
+sys.path.insert(0, os.path.dirname(TOOL))
+try:
+    import run_reference as RR
+finally:
+    sys.path.pop(0)
+REF = RR.find_reference()
+
+pytestmark = [pytest.mark.gpu,
+              pytest.mark.skipif(REF is None, reason="needs the reference project's scripts: set B200_REFERENCE_DIR")]
 
 
 def _run(*args, timeout=1500):
@@ -29,7 +37,7 @@ def _run(*args, timeout=1500):
 @pytest.fixture(scope="module")
 def reference_curve():
     res, _ = _run("overfit", "--impl", "reference", "--iters", "300", "--tf32", "0")
-    assert res["unet_module"].endswith("train/unet.py") and "_ref" in res["unet_module"] or "/root/reference" in res["unet_module"]
+    assert res["unet_module"] == os.path.join(REF, "train", "unet.py")
     return {int(k): v for k, v in res["curve"].items()}
 
 

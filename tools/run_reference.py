@@ -6,9 +6,8 @@ on top of the reference's own `train/unet.py`, for the A/B).
     python tools/run_reference.py get_metrics [--impl ...] --checkpoint models/..._best_skip.pt
 
 The scripts (reference main.py:211-325, train/overfit_check.py:36-139, train/get_metrics.py:66-173) are executed from
-their own source files -- /root/reference when it exists (this container), else the git-ignored copy under
-baseline/_ref/ that __graft_entry__.build() makes for the GPU box.  What this launcher supplies is ENVIRONMENT only
-(SURVEY.md section 8b "hazards"):
+their own source files, in the checkout of the reference project that B200_REFERENCE_DIR names (this repository does
+not ship them).  What this launcher supplies is ENVIRONMENT only (SURVEY.md section 8b "hazards"):
 
   1. sys.path: the repository root first, so `from train.unet import ...` resolves to the B200 implementation while
      `train.resnet18` / `train.overfit_check` / `train.get_metrics` (the namespace package `train` has no __init__.py)
@@ -38,30 +37,24 @@ import sys
 import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_FILES = ["main.py", "train/unet.py", "train/resnet18.py", "train/overfit_check.py", "train/get_metrics.py"]
+
+
+def find_reference() -> str | None:
+    """The absolute path of the reference checkout named by B200_REFERENCE_DIR, or None when it is unset or holds no
+    train/unet.py."""
+    cand = os.environ.get("B200_REFERENCE_DIR")
+    if cand and os.path.exists(os.path.join(cand, "train", "unet.py")):
+        return os.path.abspath(cand)
+    return None
 
 
 def reference_root() -> str:
-    """The directory holding the reference's scripts: /root/reference here, baseline/_ref on the GPU box."""
-    for cand in (os.environ.get("B200_REFERENCE_DIR"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.exists(os.path.join(cand, "train", "unet.py")):
-            return cand
-    raise RuntimeError("reference sources not found: neither /root/reference nor baseline/_ref (made by "
-                       "__graft_entry__.build() in the build container) exists")
-
-
-def stage_reference_copy() -> str | None:
-    """Copies the reference files this launcher and bench.py --impl reference execute into the git-ignored
-    baseline/_ref/ so they travel to the GPU box (where /root/reference does not exist).  Called by build()."""
-    src = "/root/reference"
-    if not os.path.exists(os.path.join(src, "train", "unet.py")):
-        return None
-    import shutil
-    dst = os.path.join(ROOT, "baseline", "_ref")
-    for f in REF_FILES:
-        os.makedirs(os.path.dirname(os.path.join(dst, f)), exist_ok=True)
-        shutil.copyfile(os.path.join(src, f), os.path.join(dst, f))
-    return dst
+    """The directory holding the reference's scripts (find_reference); raises when there is none."""
+    ref = find_reference()
+    if ref is None:
+        raise RuntimeError("reference sources not found: set B200_REFERENCE_DIR to a checkout of the reference project "
+                           "(dordanino12/unet-convlstm)")
+    return ref
 
 
 # ------------------------------------------------------------------------------------------------

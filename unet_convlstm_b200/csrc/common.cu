@@ -9,6 +9,7 @@
 
 #include <map>
 #include <mutex>
+#include <vector>
 
 namespace b200 {
 
@@ -104,6 +105,58 @@ unsigned* device_sync_counter(cudaStream_t stream) {
     unsigned* slot = pool.base + 8 * pool.used++;
     pool.by_stream[stream] = slot;
     return slot;
+}
+
+float* splitk_workspace(cudaStream_t stream, size_t floats) {
+    struct Buf {
+        float* ptr = nullptr;
+        size_t floats = 0;
+        std::vector<float*> retired;
+    };
+    static std::map<std::pair<int, cudaStream_t>, Buf> bufs;
+    static std::mutex mu;
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
+    std::lock_guard<std::mutex> lk(mu);
+    Buf& b = bufs[{dev, stream}];
+    if (b.floats < floats) {
+        // no allocation inside a CUDA-graph capture: an eager call of the same shape must size the buffer first
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(stream, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) return nullptr;
+        // the old buffer stays allocated: launches already enqueued, or captured into a graph, still use it; growing
+        // at least twofold bounds what is kept to the size of the current buffer
+        if (b.ptr) b.retired.push_back(b.ptr);
+        if (floats < 2 * b.floats) floats = 2 * b.floats;
+        b.ptr = nullptr;
+        b.floats = 0;
+        void* p = nullptr;
+        if (cudaMalloc(&p, floats * sizeof(float)) != cudaSuccess) return nullptr;
+        b.ptr = static_cast<float*>(p);
+        b.floats = floats;
+    }
+    return b.ptr;
+}
+
+__global__ void splitk_reduce_kernel(const float* __restrict__ ws, int splits, long long rows, int cols,
+                                     float* __restrict__ dw, long long ldk, int koff) {
+    const long long n = rows * cols;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+        float s = ws[i];
+        for (int k = 1; k < splits; ++k) s += ws[k * n + i];
+        const long long r = i / cols;
+        dw[r * ldk + koff + (i - r * cols)] += s;
+    }
+}
+
+int splitk_reduce(const float* ws, int splits, long long rows, int cols, float* dw, long long ldk, int koff,
+                  cudaStream_t stream) {
+    const long long n = rows * cols;
+    long long blocks = (n + 255) / 256;
+    if (blocks > 8LL * num_sms()) blocks = 8LL * num_sms();
+    splitk_reduce_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(ws, splits, rows, cols, dw, ldk, koff);
+    B200_CUDA_CHECK(cudaGetLastError());
+    return B200_OK;
 }
 
 // ----------------------------------------------------------------------------------------------

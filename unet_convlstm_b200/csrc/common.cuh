@@ -45,6 +45,15 @@ struct PerDeviceOnce {
 int* device_error_flag();  // one int in device memory, zero unless a watchdog fired
 unsigned* device_sync_counter(cudaStream_t stream);  // step counter of the timestep-persistent kernels, per (device, stream)
 
+// Split-K weight gradients without atomics, so that the result does not depend on the order in which the reduction
+// splits finish: every split stores its partial dW [rows][cols] to its own slice of a per-(device, stream) workspace,
+// then splitk_reduce adds the slices to dw[r * ldk + koff + c] in split order.
+// Grows on demand and is kept for the life of the process; nullptr if cudaMalloc fails or if it would have to grow
+// while the stream is being captured into a CUDA graph.
+float* splitk_workspace(cudaStream_t stream, size_t floats);
+int splitk_reduce(const float* ws, int splits, long long rows, int cols, float* dw, long long ldk, int koff,
+                  cudaStream_t stream);
+
 // ---- TMA tensor-map construction (driver entry point resolved at run time, no libcuda link) ----
 // Activation map over a bf16 NHWC tensor viewed as {C, W, H, B, T}; box = {box_c, Wt, Ht, Bt, 1}.
 int make_act_tmap(CUtensorMap* out, const void* base, int C, int W, int H, int B, int T, int box_c,

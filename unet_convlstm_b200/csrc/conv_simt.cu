@@ -215,7 +215,11 @@ __global__ void __launch_bounds__(256) wgrad_simt_kernel(const WgradSimtParams p
         for (int j = 0; j < 4; ++j) {
             const int n = n0 + tx * 4 + j;
             if (n >= p.Nz) continue;
-            atomicAdd(p.dw + (static_cast<long long>(tap) * p.Nz + n) * p.ldk + p.koff + c, acc[i][j]);
+            float* o = p.dw + blockIdx.z * p.split_stride + (static_cast<long long>(tap) * p.Nz + n) * p.ldk + p.koff + c;
+            if (gridDim.z > 1)
+                *o = acc[i][j];
+            else
+                *o += acc[i][j];
         }
     }
 }
@@ -231,13 +235,28 @@ int launch_wgrad_simt(WgradSimtParams p, int dtype_fp32, cudaStream_t stream) {
     if (want > 65535) want = 65535;
     p.m_per_block = ((M + want - 1) / want + 15) / 16 * 16;
     const unsigned gz = static_cast<unsigned>((M + p.m_per_block - 1) / p.m_per_block);
+    float* const dw = p.dw;
+    const long long ldk = p.ldk;
+    const int koff = p.koff;
+    p.split_stride = 0;
+    if (gz > 1) {
+        p.split_stride = static_cast<long long>(Kflat) * p.Nz;
+        p.dw = splitk_workspace(stream, gz * static_cast<size_t>(p.split_stride));
+        if (!p.dw) {
+            set_last_error("wgrad_simt: no split-K workspace (cudaMalloc failed, or growth during graph capture)");
+            return B200_ERR_CUDA;
+        }
+        p.ldk = p.Csrc;
+        p.koff = 0;
+    }
     dim3 grid(gx, gy, gz);
     if (dtype_fp32)
         wgrad_simt_kernel<float><<<grid, 256, 0, stream>>>(p);
     else
         wgrad_simt_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(p);
     B200_CUDA_CHECK(cudaGetLastError());
-    return B200_OK;
+    if (gz == 1) return B200_OK;
+    return splitk_reduce(p.dw, gz, static_cast<long long>(p.ksize) * p.ksize * p.Nz, p.Csrc, dw, ldk, koff, stream);
 }
 
 }  // namespace b200

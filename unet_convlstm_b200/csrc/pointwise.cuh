@@ -88,6 +88,7 @@ struct WgradSimtParams {
     long long ldk;
     int koff;
     long long m_per_block;
+    long long split_stride;  // with more than one pixel split: dw is the split-K workspace, split z at dw + z * split_stride
 };
 int launch_wgrad_simt(WgradSimtParams p, int dtype_fp32, cudaStream_t stream);
 

@@ -20,7 +20,7 @@
 // MMAs (kx = 0, 1, 2) per K step; the other five slots read rows past the taps and are never stored.
 //
 // Warp roles: warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue (transposed fp32
-// stores / red.global.add for split-K, as wgrad_tc.cu).
+// stores; split-K partials go to the workspace slices, as in wgrad_tc.cu).
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -43,15 +43,12 @@ struct WgradHaloParams {
     int s_tiles;       // Nz / 64
     uint32_t src_bytes, src_stage_bytes;
     int stages;        // pipeline depth that fits in shared memory (3 or 4)
-    float* dw;
+    float* dw;         // with splits > 1 the split-K workspace, split s at dw + s * split_stride
     long long ldk;
     int koff;
+    long long split_stride;
     int* err_flag;
 };
-
-__device__ __forceinline__ void wh_red_add_f32(float* addr, float a) {
-    asm volatile("red.global.add.f32 [%0], %1;" ::"l"(addr), "f"(a) : "memory");
-}
 
 __global__ void __launch_bounds__(WH_THREADS, 1)
 wgrad_halo_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constant__ CUtensorMap tm_src,
@@ -216,7 +213,7 @@ wgrad_halo_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_consta
             for (int g = 0; g < ngroups; ++g) {
                 const int tp = p.Cs == 64 ? 2 * g + gi : gi * 3 + g;
                 const bool valid = p.Cs == 64 ? tp < 9 : gi < 3;
-                float* row = p.dw + (static_cast<long long>(valid ? tp : 0) * p.Nz + s0) * p.ldk + p.koff + c;
+                float* row = p.dw + split * p.split_stride + (static_cast<long long>(valid ? tp : 0) * p.Nz + s0) * p.ldk + p.koff + c;
                 const uint32_t t_row = tmem_base + g * 64 + (uint32_t(q * 32) << 16);
 #pragma unroll 1
                 for (int c16 = 0; c16 < 4; ++c16) {
@@ -226,12 +223,7 @@ wgrad_halo_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_consta
                     if (!valid) continue;
                     float* o = row + static_cast<long long>(c16) * 16 * p.ldk;  // transposed: lanes = source channels
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        if (p.splits > 1)
-                            wh_red_add_f32(o + j * p.ldk, __uint_as_float(v[j]));
-                        else
-                            o[j * p.ldk] = __uint_as_float(v[j]);
-                    }
+                    for (int j = 0; j < 16; ++j) o[j * p.ldk] = __uint_as_float(v[j]);
                 }
             }
             tc_fence_before();
@@ -287,6 +279,16 @@ int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, 
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
     p.dw = dw; p.ldk = ldk; p.koff = koff;
+    if (p.splits > 1) {
+        p.split_stride = 9LL * Nz * Csrc;
+        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+        if (!p.dw) {
+            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+            return B200_ERR_CUDA;
+        }
+        p.ldk = Csrc;
+        p.koff = 0;
+    }
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
@@ -315,7 +317,8 @@ int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, 
     const int grid = total < nsm ? total : nsm;
     wgrad_halo_kernel<<<grid, WH_THREADS, smem, stream>>>(tz, ts, p);
     B200_CUDA_CHECK(cudaGetLastError());
-    return B200_OK;
+    if (p.splits == 1) return B200_OK;
+    return splitk_reduce(p.dw, p.splits, 9LL * Nz, Csrc, dw, ldk, koff, stream);
 }
 
 }  // namespace b200

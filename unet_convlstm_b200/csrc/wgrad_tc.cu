@@ -25,8 +25,9 @@
 //     128 dz channels would be half empty, so the roles are swapped: A = G = 128/Csrc tap-shifted
 //     source boxes stacked along M (rows = (tap, source channel)), B = dz channels (N).
 //
-// Work units = (reduction split) x (tap-group set, S tile, V tile); partial sums of different splits
-// are combined with fp32 reductions (red.global.add) into the caller's zero-initialised buffer.
+// Work units = (reduction split) x (tap-group set, S tile, V tile); with more than one split each split stores its
+// partial sums to its own workspace slice and splitk_reduce (common.cu) adds them to dw in split order, so the
+// result is the same from run to run.
 // Warp roles: warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue.
 #include "common.cuh"
 #include "ptx.cuh"
@@ -51,9 +52,10 @@ struct WgradParams {
     int GU;          // groups (accumulators) per unit
     int ngsets;      // ceil(ngroups / GU)
     int s_tiles, v_tiles, out_tiles;
-    float* dw;       // [taps][Nz][ldk]
+    float* dw;       // [taps][Nz][ldk]; with splits > 1 the split-K workspace, split s at dw + s * split_stride
     long long ldk;
     int koff;
+    long long split_stride;
     int* err_flag;
     int in_fp32;     // 1: dz and src are fp32 tensors, tcgen05 kind::tf32 (the "tf32" precision mode); a pipeline stage
                      // then holds 32 pixels instead of 64 -- the same bytes, the same four MMAs (K = 8 pixels each)
@@ -70,15 +72,6 @@ struct WgCfg {
     static constexpr int MAX_GU = 512 / BLOCK_N;
     static constexpr int SMEM_BYTES = SV * V_BYTES + SS * S_BYTES + 1024 + 256;
 };
-
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c),
-                 "f"(d)
-                 : "memory");
-}
-__device__ __forceinline__ void red_add_f32(float* addr, float a) {
-    asm volatile("red.global.add.f32 [%0], %1;" ::"l"(addr), "f"(a) : "memory");
-}
 
 struct WgUnit {
     int split, gset, s0, v0, scols, vcols, ngr;
@@ -386,11 +379,11 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constant
                     const int gi = r / p.Csrc, c = r - gi * p.Csrc;
                     const int tp = grp * p.G + gi;
                     valid = tp < p.taps;
-                    row = p.dw + (static_cast<long long>(tp) * p.Nz + u.s0) * p.ldk + p.koff + c;
+                    row = p.dw + u.split * p.split_stride + (static_cast<long long>(tp) * p.Nz + u.s0) * p.ldk + p.koff + c;
                 } else {
                     const int n = u.s0 + r;
                     valid = n < p.Nz;
-                    row = p.dw + (static_cast<long long>(grp) * p.Nz + n) * p.ldk + p.koff + u.v0;
+                    row = p.dw + u.split * p.split_stride + (static_cast<long long>(grp) * p.Nz + n) * p.ldk + p.koff + u.v0;
                 }
                 const uint32_t t_row = tmem_base + g * BLOCK_N + (uint32_t(q * 32) << 16);
 #pragma unroll 1
@@ -403,26 +396,14 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constant
                         // transposed store: consecutive lanes hold consecutive source channels
                         float* o = row + static_cast<long long>(c16) * 16 * p.ldk;
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            if (p.splits > 1)
-                                red_add_f32(o + j * p.ldk, __uint_as_float(v[j]));
-                            else
-                                o[j * p.ldk] = __uint_as_float(v[j]);
-                        }
+                        for (int j = 0; j < 16; ++j) o[j * p.ldk] = __uint_as_float(v[j]);
                     } else {
                         float* o = row + c16 * 16;
-                        if (p.splits > 1) {
 #pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                red_add_v4(o + 4 * j, __uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                           __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                        } else {
-#pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                reinterpret_cast<float4*>(o)[j] =
-                                    make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                                __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                        }
+                        for (int j = 0; j < 4; ++j)
+                            reinterpret_cast<float4*>(o)[j] =
+                                make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
+                                            __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
                     }
                 }
             }
@@ -540,6 +521,16 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
     p.dw = dw; p.ldk = ldk; p.koff = koff;
+    if (p.splits > 1) {
+        p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
+        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+        if (!p.dw) {
+            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+            return B200_ERR_CUDA;
+        }
+        p.ldk = Csrc;
+        p.koff = 0;
+    }
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
@@ -549,16 +540,19 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
     if (rc != B200_OK) return rc;
     if (stacked) {
         switch (block_n) {
-            case 256: return launch_wgrad_impl<256, true>(tz, ts, p, stream);
-            case 128: return launch_wgrad_impl<128, true>(tz, ts, p, stream);
-            default: return launch_wgrad_impl<64, true>(tz, ts, p, stream);
+            case 256: rc = launch_wgrad_impl<256, true>(tz, ts, p, stream); break;
+            case 128: rc = launch_wgrad_impl<128, true>(tz, ts, p, stream); break;
+            default: rc = launch_wgrad_impl<64, true>(tz, ts, p, stream); break;
+        }
+    } else {
+        switch (block_n) {
+            case 256: rc = launch_wgrad_impl<256, false>(tz, ts, p, stream); break;
+            case 128: rc = launch_wgrad_impl<128, false>(tz, ts, p, stream); break;
+            default: rc = launch_wgrad_impl<64, false>(tz, ts, p, stream); break;
         }
     }
-    switch (block_n) {
-        case 256: return launch_wgrad_impl<256, false>(tz, ts, p, stream);
-        case 128: return launch_wgrad_impl<128, false>(tz, ts, p, stream);
-        default: return launch_wgrad_impl<64, false>(tz, ts, p, stream);
-    }
+    if (rc != B200_OK || p.splits == 1) return rc;
+    return splitk_reduce(p.dw, p.splits, static_cast<long long>(p.taps) * Nz, Csrc, dw, ldk, koff, stream);
 }
 
 }  // namespace b200

@@ -19,7 +19,8 @@
 // Pipeline (barriers at the same shared-memory offset in both CTAs): sfull / vfull live in the leader (two
 // arrive.expect_tx, both CTAs' cta_group::2 TMA copies complete on them); sempty / vempty / tfull are signalled in
 // both CTAs by the leader's multicast tcgen05.commit; tempty collects the epilogue warps of the pair.  Work units,
-// reduction splits, the five producer warps and the transposed fp32 red.add epilogue are those of wgrad_tc.cu.
+// reduction splits (with their workspace slices), the five producer warps and the transposed fp32 store epilogue are
+// those of wgrad_tc.cu.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -44,9 +45,10 @@ struct Wgrad2Params {
     int ngroups, GU, ngsets;
     int gset_inner;             // unit order: tap sets fastest (1) or slowest (0)
     int s_tiles, v_tiles, out_tiles;
-    float* dw;
+    float* dw;                  // with splits > 1 the split-K workspace, split s at dw + s * split_stride
     long long ldk;
     int koff;
+    long long split_stride;
     int* err_flag;
 };
 
@@ -61,13 +63,6 @@ struct Wg2Cfg {
     static constexpr int MAX_GU = 512 / BLOCK_N;
     static constexpr int SMEM_BYTES = SV * V_BYTES + SS * S_BYTES + 1024 + 512;
 };
-
-__device__ __forceinline__ void w2_red_add_f32(float* addr, float a) {
-    asm volatile("red.global.add.f32 [%0], %1;" ::"l"(addr), "f"(a) : "memory");
-}
-__device__ __forceinline__ void w2_red_add_v4(float* addr, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
 
 struct Wg2Unit {
     int split, gset, s0, v0, ngr;
@@ -355,12 +350,12 @@ wgrad_tc2_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constan
                     const int gi = r / p.Csrc, c = r - gi * p.Csrc;
                     const int tp = (grp * 2 + static_cast<int>(rank)) * p.G + gi;
                     valid = tp < p.taps;
-                    row = p.dw + (static_cast<long long>(valid ? tp : 0) * p.Nz + u.s0) * p.ldk + p.koff + c;
+                    row = p.dw + u.split * p.split_stride + (static_cast<long long>(valid ? tp : 0) * p.Nz + u.s0) * p.ldk + p.koff + c;
                 } else {
                     // row r of this CTA = dz channel; column = source channel
                     const int n = u.s0 + static_cast<int>(rank) * W2_BLOCK_M + r;
                     valid = n < p.Nz;
-                    row = p.dw + (static_cast<long long>(grp) * p.Nz + (valid ? n : 0)) * p.ldk + p.koff + u.v0;
+                    row = p.dw + u.split * p.split_stride + (static_cast<long long>(grp) * p.Nz + (valid ? n : 0)) * p.ldk + p.koff + u.v0;
                 }
                 const uint32_t t_row = tmem_base + g * BLOCK_N + (uint32_t(q * 32) << 16);
 #pragma unroll 1
@@ -373,26 +368,14 @@ wgrad_tc2_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constan
                         // transposed store: consecutive lanes hold consecutive source channels
                         float* o = row + static_cast<long long>(c16) * 16 * p.ldk;
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            if (p.splits > 1)
-                                w2_red_add_f32(o + j * p.ldk, __uint_as_float(v[j]));
-                            else
-                                o[j * p.ldk] = __uint_as_float(v[j]);
-                        }
+                        for (int j = 0; j < 16; ++j) o[j * p.ldk] = __uint_as_float(v[j]);
                     } else {
                         float* o = row + c16 * 16;
-                        if (p.splits > 1) {
 #pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                w2_red_add_v4(o + 4 * j, __uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                              __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                        } else {
-#pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                reinterpret_cast<float4*>(o)[j] =
-                                    make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                                __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                        }
+                        for (int j = 0; j < 4; ++j)
+                            reinterpret_cast<float4*>(o)[j] =
+                                make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
+                                            __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
                     }
                 }
             }
@@ -505,6 +488,16 @@ int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, i
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
     p.dw = dw; p.ldk = ldk; p.koff = koff;
+    if (p.splits > 1) {
+        p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
+        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+        if (!p.dw) {
+            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+            return B200_ERR_CUDA;
+        }
+        p.ldk = Csrc;
+        p.koff = 0;
+    }
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
@@ -514,16 +507,19 @@ int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, i
     if (rc != B200_OK) return rc;
     if (stacked) {
         switch (block_n) {
-            case 256: return launch_wgrad2_impl<256, true>(tz, ts, p, stream);
-            case 128: return launch_wgrad2_impl<128, true>(tz, ts, p, stream);
-            default: return launch_wgrad2_impl<64, true>(tz, ts, p, stream);
+            case 256: rc = launch_wgrad2_impl<256, true>(tz, ts, p, stream); break;
+            case 128: rc = launch_wgrad2_impl<128, true>(tz, ts, p, stream); break;
+            default: rc = launch_wgrad2_impl<64, true>(tz, ts, p, stream); break;
+        }
+    } else {
+        switch (block_n) {
+            case 256: rc = launch_wgrad2_impl<256, false>(tz, ts, p, stream); break;
+            case 128: rc = launch_wgrad2_impl<128, false>(tz, ts, p, stream); break;
+            default: rc = launch_wgrad2_impl<64, false>(tz, ts, p, stream); break;
         }
     }
-    switch (block_n) {
-        case 256: return launch_wgrad2_impl<256, false>(tz, ts, p, stream);
-        case 128: return launch_wgrad2_impl<128, false>(tz, ts, p, stream);
-        default: return launch_wgrad2_impl<64, false>(tz, ts, p, stream);
-    }
+    if (rc != B200_OK || p.splits == 1) return rc;
+    return splitk_reduce(p.dw, p.splits, static_cast<long long>(p.taps) * Nz, Csrc, dw, ldk, koff, stream);
 }
 
 }  // namespace b200
