@@ -5,7 +5,8 @@
  * names the reference lines whose arithmetic it replaces.  Conventions:
  *   - every pointer is a device pointer owned by the caller (the multi-tensor entry points take HOST arrays of
  *     device pointers and say so); nothing is allocated or freed here except one 4-byte watchdog flag per device
- *     and one 4-byte step counter per (device, stream) that runs a timestep-persistent kernel;
+ *     and one 4-byte step counter per (device, stream) that runs a timestep-persistent kernel, and the split-K
+ *     workspace per (device, stream) of the split weight gradients and b200_*_splitk_tc (kept for the process);
  *   - calls on distinct streams may be made concurrently from different threads;
  *   - activations are NHWC ("channels last"), bf16 on the tensor-core path (*_tc), fp32 or bf16 on
  *     the generic SIMT path; a sequence tensor is [T][B][H][W][C];
@@ -89,6 +90,27 @@ int b200_convlstm_cell_fwd_tc(const void* x, int Cin, const void* h_prev, int Ch
 int b200_convlstm_seq_fwd_tc(const void* x_seq, int Cin, void* h_all, int Ch, int T, int B, int H, int W,
                              const void* wpacked, const float* bias_packed, float* c_all, void* gates,
                              int have_h0, int ksize, void* stream);
+
+/* ---- Split K for single-frame problems with few M tiles (streaming inference, one frame at a time: at B = 1 and
+ * 4x4 .. 16x16 pixels the tensor-core tiling has a single M tile, so the unsplit launch occupies a handful of SMs and
+ * each CTA walks the whole K = 9 x (C0 + C1) loop alone).  The implicit GEMM of b200_conv_tc_fwd (1-CTA kernel) runs
+ * `splits` contiguous ranges of its (tap, 64-channel chunk) k-blocks side by side; each range stores fp32 partial sums
+ * [P][N] (P = B*H*W) to its own slice of a library-owned per-(device, stream) workspace, and a second kernel adds the
+ * slices in split order -- no atomics, the result does not depend on which split finishes first -- and applies the
+ * epilogue.  Two kernel launches per call.  The workspace grows on the first call of a larger shape on a stream and
+ * never during a CUDA-graph capture (that call fails instead).  bf16 only.
+ * b200_splitk_splits: the number of splits the library recommends for a bf16 convolution of that shape (1 = do not
+ * split; see csrc/capi.cu for the rule and the measurement behind it). */
+int b200_splitk_splits(int B, int H, int W, int C0, int C1, int N, int ksize);
+/* b200_convlstm_cell_fwd_tc split over K: arguments as there, without gates_out (inference keeps no gates). */
+int b200_convlstm_cell_fwd_splitk_tc(const void* x, int Cin, const void* h_prev, int Ch, int B, int H, int W,
+                                     const void* wpacked, const float* bias_packed, const float* c_prev, float* c_next,
+                                     void* h_next, int splits, int ksize, void* stream);
+/* b200_conv_affine_relu_tc_fwd of one frame (T = 1) split over K: dst = relu?(conv * scale + shift), bf16 or fp32
+ * (out_fp32); scale / shift may be NULL (1 / 0), which leaves the plain convolution. */
+int b200_conv_affine_relu_splitk_tc(const void* src0, int C0, const void* src1, int C1, int B, int H, int W,
+                                    const void* wpacked, const float* scale, const float* shift, int N, int ksize,
+                                    void* dst, int out_fp32, int relu, int splits, void* stream);
 
 /* ---- "tf32" precision mode (north_star: "bf16/TF32 inputs with fp32 accumulation"; the reference's own GPU numerics:
  * torch enables TF32 in cuDNN convolutions by default).  Same implicit GEMM as the *_tc entry points with fp32 tensors

@@ -278,24 +278,19 @@ class TemporalUNetDualView(nn.Module):
         xb, skips = self._encode(_to_nhwc(x_t, _in_pad(x_t.shape[1])))
         return _to_nchw(xb), tuple(_to_nchw(s) for s in skips)
 
-    def forward(self, x_seq, state=None):
-        _require_cuda(x_seq, "TemporalUNetDualView")
-        B, T, C, H, W = x_seq.shape
-        act = ops.act_dtype()
-        # [B,T,C,H,W] fp32 -> [T,B,H,W,C] channels-last (input channels zero-padded in bf16 mode)
-        x = Fn.permute_cast(x_seq, (1, 0, 3, 4, 2), act, _in_pad(C))
+    def _core(self, x, st, skip_st=None):
+        """x [T,B,H,W,C] channels-last in the activation dtype -> (y fp32 [T,B,H,W,out], final (h, c) of every temporal
+        layer, final (h, c) of lstm_skip3 and lstm_skip2).  st: initial NHWC state per temporal layer (or None);
+        skip_st: the skip cells' initial states [(h, c) of lstm_skip3, (h, c) of lstm_skip2], None = zero (forward)."""
         xb, (x3, x2, x1, x0) = self._encode(x)
-
-        st = None
-        if state is not None:
-            st = [None if s is None or s[0] is None else
-                  (Fn.permute_cast(s[0], (0, 2, 3, 1), act), Fn.permute_cast(s[1], (0, 2, 3, 1), torch.float32))
-                  for s in state]
         hb, finals = self.temporal._seq(xb, st)
+        skip_finals = []
         if self.use_skip_lstm:
-            # skip LSTMs always start from a zero state and their final state is dropped (unet.py:190-191)
-            x3, _ = self.lstm_skip3._seq(x3, None)
-            x2, _ = self.lstm_skip2._seq(x2, None)
+            # forward: the skip LSTMs always start from a zero state and their final state is dropped (unet.py:190-191);
+            # streaming inference (FrameStream) carries it from frame to frame
+            x3, f3 = self.lstm_skip3._seq(x3, None if skip_st is None else [skip_st[0]])
+            x2, f2 = self.lstm_skip2._seq(x2, None if skip_st is None else [skip_st[1]])
+            skip_finals = f3 + f2
 
         d3 = self.up3._seq(hb, x3)
         d2 = self.up2._seq(d3, x2)
@@ -303,6 +298,15 @@ class TemporalUNetDualView(nn.Module):
         # the last DoubleConv and the 1x1 output convolution: fp32 [T,B,H,W,out]; with one output channel the normalise
         # pass of the DoubleConv produces it directly (the 64-channel full-resolution activation is never written)
         y = self.up0._seq(d1, x0, self.outc.conv)
+        return y, finals, skip_finals
+
+    def forward(self, x_seq, state=None):
+        _require_cuda(x_seq, "TemporalUNetDualView")
+        B, T, C, H, W = x_seq.shape
+        act = ops.act_dtype()
+        # [B,T,C,H,W] fp32 -> [T,B,H,W,C] channels-last (input channels zero-padded in bf16 mode)
+        x = Fn.permute_cast(x_seq, (1, 0, 3, 4, 2), act, _in_pad(C))
+        y, finals, _ = self._core(x, None if state is None else _state_to_nhwc(state, act))
 
         # list of T frames as views of one buffer.  unbind, not T x select: the backward of unbind stacks the T frame
         # gradients in one pass; T selects each materialise a full-size zero tensor that autograd then adds up
@@ -311,9 +315,26 @@ class TemporalUNetDualView(nn.Module):
             out_seq = list(y.view(T, B, 1, H, W).unbind(0))  # C == 1: NHWC and NCHW coincide
         else:
             out_seq = list(Fn.permute_cast(y, (0, 1, 4, 2, 3), torch.float32).unbind(0))
-        new_state = [(Fn.permute_cast(h, (0, 3, 1, 2), torch.float32), Fn.permute_cast(c, (0, 3, 1, 2), torch.float32))
-                     for h, c in finals]
-        return out_seq, new_state
+        return out_seq, _state_to_nchw(finals)
+
+    def stream(self, state=None):
+        """Streaming inference, one frame at a time with every ConvLSTM state carried (unet_convlstm_b200/stream.py):
+        for an eval-mode model under no_grad, [s.step(x[:, t]) for t in range(T)] and s.state equal model(x, state)."""
+        from unet_convlstm_b200.stream import FrameStream
+        return FrameStream(self, state)
+
+
+def _state_to_nhwc(state, act):
+    """forward's `state` ([(h, c)] NCHW per temporal layer, entries may be None) -> NHWC (h: act dtype, c: fp32)."""
+    return [None if s is None or s[0] is None else
+            (Fn.permute_cast(s[0], (0, 2, 3, 1), act), Fn.permute_cast(s[1], (0, 2, 3, 1), torch.float32))
+            for s in state]
+
+
+def _state_to_nchw(finals):
+    """[(h, c)] NHWC -> the [(h, c)] NCHW fp32 state forward returns."""
+    return [(Fn.permute_cast(h, (0, 3, 1, 2), torch.float32), Fn.permute_cast(c, (0, 3, 1, 2), torch.float32))
+            for h, c in finals]
 
 
 # -----------------------------------------------------------------------------------------------

@@ -53,6 +53,7 @@ _protos = None
 CALLS: dict = {}
 # device kernels launched per call of each entry point (memsets are not counted)
 KERNELS_PER_CALL = {
+    "b200_convlstm_cell_fwd_splitk_tc": 2, "b200_conv_affine_relu_splitk_tc": 2,
     "b200_conv_tc_fwd": 1, "b200_conv_bnstats_tc_fwd": 1, "b200_convT2x2_tc_fwd": 1, "b200_conv_affine_relu_tc_fwd": 1, "b200_convlstm_cell_fwd_tc": 1, "b200_convlstm_seq_fwd_tc": 1, "b200_convlstm_seq_bwd_tc": 1, "b200_wgrad_tc": 1, "b200_conv_simt_fwd": 1,
     "b200_wgrad_simt": 1, "b200_bn_stats": 1, "b200_bn_finalize": 1, "b200_bn_relu_apply": 1,
     "b200_bn_relu_bwd_reduce": 1, "b200_bn_bwd_finalize": 1, "b200_bn_relu_bwd_apply": 1,

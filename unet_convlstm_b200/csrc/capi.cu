@@ -212,6 +212,87 @@ extern "C" int b200_convlstm_seq_fwd_tc(const void* x_seq, int Cin, void* h_all,
 }
 
 // ------------------------------------------------------------------------------------------------
+// Split K for single-frame GEMMs with few M tiles (streaming inference, unet_convlstm_b200/stream.py)
+// ------------------------------------------------------------------------------------------------
+// Rule (b200_splitk_splits): split only when the 1-CTA tiling has at most SPLITK_MAX_M_TILES M tiles and all its
+// tiles together occupy at most 1 / SPLITK_SM_SHARE of the SMs; then S = SMs / tiles (about one wave of tiles x S
+// CTAs), capped so that every split keeps at least SPLITK_MIN_KB k-blocks (one k-block = one tap x 64 channels).
+// Measured on a B200 at 1000 W (tools/bench_infer.py --stream, profiles/stream_infer_b200.txt): the split cell and
+// folded convs of the 4x4 / 8x8 / 16x16 levels at B = 1 and 8 run 1.3-2.1x faster than the unsplit launch; below
+// ~16 k-blocks per split the cell loses again (8x8 Ch 512, B = 1: S = 8 1.61x, S = 16 1.39x; 16x16 Ch 256: S = 4
+// 1.30x, S = 8 1.20x; at B = 8 S = 16 falls to 0.27-0.60x), so 16 is the minimum -- within ~5 % of the best S at
+// every measured shape.  Shapes with more M tiles (16x16 at B = 8, every level at B = 64) were not measured split
+// and stay unsplit.
+static constexpr int SPLITK_MAX_M_TILES = 4;
+static constexpr int SPLITK_SM_SHARE = 4;
+static constexpr int SPLITK_MIN_KB = 16;
+
+extern "C" int b200_splitk_splits(int B, int H, int W, int C0, int C1, int N, int ksize) {
+    MTile mt;
+    if (!plan_mtile(B, H, W, 128, &mt) || C0 <= 0 || C0 % 16 != 0 || C1 % 16 != 0 || (ksize & 1) == 0) return 1;
+    const int block_n = pick_block_n(N, EPI_STORE);
+    if (block_n == 0) return 1;
+    const int m_tiles = mt.tiles_w * mt.tiles_h * mt.tiles_b;
+    const int tiles = m_tiles * ((N + block_n - 1) / block_n);
+    if (m_tiles > SPLITK_MAX_M_TILES || tiles * SPLITK_SM_SHARE > num_sms()) return 1;
+    int s = num_sms() / tiles;
+    const int by_k = conv_tc_num_kb(C0, C1, ksize) / SPLITK_MIN_KB;
+    if (s > by_k) s = by_k;
+    return s >= 2 ? s : 1;
+}
+
+static float* splitk_ws_or_error(const char* who, cudaStream_t st, int splits, long long P, int N) {
+    float* ws = splitk_workspace(st, static_cast<size_t>(splits) * P * N);
+    if (!ws)
+        set_last_error("%s: no split-K workspace (cudaMalloc failed, or it would have to grow during a CUDA-graph "
+                       "capture: run the same shape once on this stream before capturing)", who);
+    return ws;
+}
+
+extern "C" int b200_convlstm_cell_fwd_splitk_tc(const void* x, int Cin, const void* h_prev, int Ch, int B, int H, int W,
+                                                const void* wpacked, const float* bias_packed, const float* c_prev,
+                                                float* c_next, void* h_next, int splits, int ksize, void* stream) {
+    if (!x || !wpacked || !c_next || !h_next || Ch <= 0 || Cin <= 0 || splits < 1 || (ksize & 1) == 0) {
+        set_last_error("b200_convlstm_cell_fwd_splitk_tc: bad arguments");
+        return B200_ERR_ARG;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ConvTcParams p = {};
+    p.T = 1; p.B = B; p.H = H; p.W = W;
+    p.C0 = Cin; p.C1 = h_prev ? Ch : 0;   // zero state: the h half of K is skipped, as in the unsplit cell
+    p.N = 4 * Ch; p.ksize = ksize;
+    p.wK = Cin + Ch;
+    const long long P = static_cast<long long>(B) * H * W;
+    float* ws = splitk_ws_or_error("b200_convlstm_cell_fwd_splitk_tc", st, splits, P, p.N);
+    if (!ws) return B200_ERR_CUDA;
+    int S = 0;
+    int rc = launch_conv_tc_splitk(x, h_prev, wpacked, p, splits, ws, &S, st);
+    if (rc != B200_OK) return rc;
+    const int cht = Ch % 64 == 0 ? 64 : (Ch % 32 == 0 ? 32 : 16);   // the gate interleave of b200_pack_weight
+    return launch_splitk_lstm_cell(ws, S, P, Ch, cht, bias_packed, c_prev, c_next, h_next, st);
+}
+
+extern "C" int b200_conv_affine_relu_splitk_tc(const void* src0, int C0, const void* src1, int C1, int B, int H, int W,
+                                               const void* wpacked, const float* scale, const float* shift, int N,
+                                               int ksize, void* dst, int out_fp32, int relu, int splits, void* stream) {
+    if (!src0 || !wpacked || !dst || N <= 0 || splits < 1 || (ksize & 1) == 0 || (C1 > 0 && !src1)) {
+        set_last_error("b200_conv_affine_relu_splitk_tc: bad arguments");
+        return B200_ERR_ARG;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ConvTcParams p = {};
+    p.T = 1; p.B = B; p.H = H; p.W = W;
+    p.C0 = C0; p.C1 = C1; p.N = N; p.ksize = ksize;
+    const long long P = static_cast<long long>(B) * H * W;
+    float* ws = splitk_ws_or_error("b200_conv_affine_relu_splitk_tc", st, splits, P, N);
+    if (!ws) return B200_ERR_CUDA;
+    int S = 0;
+    int rc = launch_conv_tc_splitk(src0, src1, wpacked, p, splits, ws, &S, st);
+    if (rc != B200_OK) return rc;
+    return launch_splitk_affine(ws, S, P, N, scale, shift, relu, dst, out_fp32, st);
+}
+
+// ------------------------------------------------------------------------------------------------
 // "tf32" precision mode: fp32 tensors, tcgen05 kind::tf32 products, fp32 accumulation
 // ------------------------------------------------------------------------------------------------
 extern "C" int b200_conv_tf32_supported(int B, int H, int W, int C0, int C1, int N, int lstm) {

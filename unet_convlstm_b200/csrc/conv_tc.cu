@@ -123,6 +123,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
     const int chunks1 = p.C1 / p.kc;
     const int chunks = chunks0 + chunks1;
     const int num_kb = taps * chunks;
+    // K range of this CTA (split K, see ConvTcParams::kb_split): k-blocks [kb_lo, kb_hi) of the (tap, chunk) loop
+    const int kb_lo = p.kb_split > 0 ? static_cast<int>(blockIdx.z) * p.kb_split : 0;
+    const int kb_hi = p.kb_split > 0 ? min(kb_lo + p.kb_split, num_kb) : num_kb;
     const int total_tiles = p.num_m_tiles * p.num_n_tiles;
     // timestep-persistent mode (EPI_LSTM only): the kernel iterates over the whole sequence, h_t and
     // c_t stay in the L2-resident state buffers and a grid-wide counter separates the steps
@@ -208,11 +211,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                 TileCoord tc = decode_tile(p, tile, BLOCK_N);
                 if (seq) tc.t = step_t(step);
                 if (!tile_active(tc.t, tc.n0)) continue;
-                int ky = 0, kx = 0;
+                int ky = 0, kx = 0, kbi = 0;
                 for (int tap = 0; tap < taps; ++tap) {
                     const int cw = tc.w0 + kx - p.pad, chh = tc.h0 + ky - p.pad;
                     int kofs = 0;
-                    for (int c = 0; c < chunks_t; ++c, kofs += p.kc) {
+                    for (int c = 0; c < chunks_t; ++c, kofs += p.kc, ++kbi) {
+                        if (kbi < kb_lo || kbi >= kb_hi) continue;  // outside this split's K range (warp-uniform)
                         mbar_wait(empty_bar(stage), phase ^ 1u, p.err_flag, 1000 + 100 + stage);
                         if (elect_one()) {
                             const uint32_t fb = full_bar(stage);
@@ -258,7 +262,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
         const uint32_t a_lo0 = a_lo;
         constexpr uint32_t STAGE_LO = Cfg::STAGE_BYTES >> 4, B_LO = Cfg::A_BYTES >> 4;
         for (int step = 0; step < nsteps; ++step) {
-            const int num_kb_t = (seq && step == 0 && !p.seq_have_h0) ? taps * chunks0 : num_kb;
+            const int num_kb_t = min(kb_hi, (seq && step == 0 && !p.seq_have_h0) ? taps * chunks0 : num_kb);
             for (int ti = 0;; ++ti) {
                 const int tile = tile_at(ti);
                 if (tile == -2) break;
@@ -270,7 +274,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + acc * BLOCK_N;
                 uint32_t accum = 0;
-                for (int kb = 0; kb < num_kb_t; ++kb) {
+                for (int kb = kb_lo; kb < num_kb_t; ++kb) {
                     mbar_wait(full_bar(stage), phase, p.err_flag, 1000 + 200 + stage);
                     tc_fence_after();
                     if (elect_one()) {
@@ -448,7 +452,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant_
                             continue;
                         }
                         const bool second = ncol >= p.split;
-                        const long long off = second ? pix * p.ld1 + (ncol - p.split) : pix * p.ld0 + ncol;
+                        const long long off = second ? pix * p.ld1 + (ncol - p.split)
+                                                     : pix * p.ld0 + ncol + blockIdx.z * p.split_stride;
                         void* base = second ? p.dst1 : p.dst0;
                         if (p.out_fp32) {
                             float4* o = reinterpret_cast<float4*>(static_cast<float*>(base) + off);
@@ -734,7 +739,7 @@ int pick_block_n(int N, int epi) {
 
 template <int BLOCK_N, int EPI>
 static int launch_impl(const CUtensorMap& ta0, const CUtensorMap& ta1, const CUtensorMap& tb,
-                       const ConvTcParams& p, cudaStream_t stream) {
+                       const ConvTcParams& p, cudaStream_t stream, int splits = 1) {
     using Cfg = TcCfg<BLOCK_N>;
     auto kern = conv_tc_kernel<BLOCK_N, EPI>;
     static PerDeviceOnce attr_once;  // kernel attributes are per device
@@ -753,9 +758,38 @@ static int launch_impl(const CUtensorMap& ta0, const CUtensorMap& ta1, const CUt
                                                     dim3(EpiCfg<EPI>::THREADS), args, Cfg::SMEM_BYTES, stream));
         return B200_OK;
     }
-    kern<<<grid, EpiCfg<EPI>::THREADS, Cfg::SMEM_BYTES, stream>>>(ta0, ta1, tb, p);
+    kern<<<dim3(grid, 1, splits), EpiCfg<EPI>::THREADS, Cfg::SMEM_BYTES, stream>>>(ta0, ta1, tb, p);
     B200_CUDA_CHECK(cudaGetLastError());
     return B200_OK;
+}
+
+// K-block width: the widest of 128 / 64 / 32-byte rows that divides both channel counts (0: none does)
+static int pick_kc(int C0, int C1, int esize) {
+    const int kc_max = 128 / esize, kc_min = 32 / esize;
+    int kc = kc_max;
+    while (kc >= kc_min && ((C0 % kc) != 0 || (C1 % kc) != 0)) kc >>= 1;
+    return (kc < kc_min || C0 <= 0) ? 0 : kc;
+}
+
+int conv_tc_num_kb(int C0, int C1, int ksize) {
+    const int kc = pick_kc(C0, C1, 2);
+    return kc ? ksize * ksize * (C0 / kc + C1 / kc) : 0;
+}
+
+int launch_conv_tc_splitk(const void* src0, const void* src1, const void* wpacked, ConvTcParams p, int splits,
+                          float* ws, int* splits_out, cudaStream_t stream) {
+    const int num_kb = conv_tc_num_kb(p.C0, p.C1, p.ksize);
+    if (num_kb == 0 || splits < 1 || p.seq_T > 0 || p.in_fp32) {
+        set_last_error("conv_tc_splitk: bf16 single-step problems with channel counts in multiples of 16 only");
+        return B200_ERR_SHAPE;
+    }
+    p.kb_split = (num_kb + splits - 1) / splits;
+    *splits_out = (num_kb + p.kb_split - 1) / p.kb_split;  // no empty split
+    p.split_stride = static_cast<long long>(p.T) * p.B * p.H * p.W * p.N;
+    p.dst0 = ws; p.ld0 = p.N; p.split = p.N; p.dst1 = nullptr; p.ld1 = 0;
+    p.out_fp32 = 1; p.relu = 0; p.accumulate = 0;
+    p.bias = nullptr; p.scale = nullptr; p.stat_sum = nullptr; p.stat_sumsq = nullptr; p.shuf_C = 0;
+    return launch_conv_tc(src0, src1, wpacked, p, EPI_STORE, stream);
 }
 
 int launch_convlstm_seq_tc(const void* x_seq, const void* h_all, const void* wpacked, ConvTcParams p,
@@ -789,13 +823,17 @@ int launch_conv_tc(const void* src0, const void* src1, const void* wpacked, Conv
     }
     const int Ct = p.wK > 0 ? p.wK : p.C0 + p.C1;
     const int esize = p.in_fp32 ? 4 : 2;
-    const int kc_max = 128 / esize, kc_min = 32 / esize;   // K-block rows of 128 .. 32 bytes
-    int kc = kc_max;
-    while (kc >= kc_min && ((p.C0 % kc) != 0 || (p.C1 % kc) != 0)) kc >>= 1;
-    if (kc < kc_min || p.C0 <= 0) {
-        set_last_error("conv_tc: channel counts C0=%d C1=%d are not multiples of %d", p.C0, p.C1, kc_min);
+    const int kc = pick_kc(p.C0, p.C1, esize);   // K-block rows of 128 .. 32 bytes
+    if (kc == 0) {
+        set_last_error("conv_tc: channel counts C0=%d C1=%d are not multiples of %d", p.C0, p.C1, 32 / esize);
         return B200_ERR_SHAPE;
     }
+    if (p.kb_split > 0 && (epi != EPI_STORE || p.seq_T > 0 || !p.out_fp32 || p.bias || p.scale || p.relu ||
+                           p.accumulate || p.stat_sum || p.shuf_C > 0 || p.split != p.N)) {
+        set_last_error("conv_tc: split K stores plain fp32 partial sums (no bias, scale, relu, statistics or shuffle)");
+        return B200_ERR_ARG;
+    }
+    const int splits = p.kb_split > 0 ? (p.ksize * p.ksize * (p.C0 / kc + p.C1 / kc) + p.kb_split - 1) / p.kb_split : 1;
     if (p.in_fp32 && (epi == EPI_LSTM_BWD || p.seq_T > 0 || p.stat_sum || p.shuf_C > 0 || !(p.out_fp32 || epi == EPI_LSTM))) {
         set_last_error("conv_tc: the tf32 mode covers plain fp32-output convolutions and the single-step fused cell");
         return B200_ERR_ARG;
@@ -858,9 +896,9 @@ int launch_conv_tc(const void* src0, const void* src1, const void* wpacked, Conv
         }
     }
     switch (block_n) {
-        case 256: return launch_impl<256, EPI_STORE>(ta0, ta1, tb, p, stream);
-        case 128: return launch_impl<128, EPI_STORE>(ta0, ta1, tb, p, stream);
-        default: return launch_impl<64, EPI_STORE>(ta0, ta1, tb, p, stream);
+        case 256: return launch_impl<256, EPI_STORE>(ta0, ta1, tb, p, stream, splits);
+        case 128: return launch_impl<128, EPI_STORE>(ta0, ta1, tb, p, stream, splits);
+        default: return launch_impl<64, EPI_STORE>(ta0, ta1, tb, p, stream, splits);
     }
 }
 

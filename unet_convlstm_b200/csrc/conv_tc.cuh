@@ -36,6 +36,11 @@ struct ConvTcParams {
     int accumulate;      // fp32 only: dst += value
     const float* bias;   // [N] (packed order) or nullptr
     const float* scale;  // [N] or nullptr: out = acc * scale + bias (eval-mode BatchNorm folded into the conv)
+    // split K (EPI_STORE, fp32 output, no bias / scale / relu): split z = blockIdx.z accumulates the k-blocks
+    // [z * kb_split, (z + 1) * kb_split) of the (tap, channel chunk) loop and stores its partial sums at
+    // dst0 + z * split_stride.  kb_split = 0: the whole K loop, one split (every other launch).
+    int kb_split;
+    long long split_stride;
     // fused 2x2 pixel shuffle (ConvTranspose2d k=2 s=2 as a GEMM, unet.py:90-97; bf16 output, dst0 only):
     // column n = tap * shuf_C + co of input pixel (img, h, w) goes to output pixel
     // (2h + tap/2 + shuf_oy, 2w + tap%2 + shuf_ox) of a [IMG][shuf_Hd][shuf_Wd][shuf_C] tensor; bias is [shuf_C]
@@ -72,6 +77,14 @@ struct ConvTcParams {
 // Launches the kernel for one problem.  All pointers are device pointers; maps are built per call.
 int launch_conv_tc(const void* src0, const void* src1, const void* wpacked, ConvTcParams p, int epi,
                    cudaStream_t stream);
+
+// Split-K form of launch_conv_tc (1-CTA kernel, EPI_STORE): `splits` K ranges of whole k-blocks, one per
+// blockIdx.z, each storing fp32 partial sums [P][N] (P = T*B*H*W) to ws + z * P * N.  Returns the number of
+// splits actually launched (every split gets at least one k-block) in *splits_out.
+int launch_conv_tc_splitk(const void* src0, const void* src1, const void* wpacked, ConvTcParams p, int splits,
+                          float* ws, int* splits_out, cudaStream_t stream);
+// k-blocks of the implicit GEMM over [src0 ; src1] (taps x channel chunks), as launch_conv_tc will tile it.
+int conv_tc_num_kb(int C0, int C1, int ksize);
 
 // Whole-sequence forward of one ConvLSTM layer in ONE cooperative launch (see ConvTcParams::seq_T).
 int launch_convlstm_seq_tc(const void* x_seq, const void* h_all, const void* wpacked, ConvTcParams p,

@@ -1898,4 +1898,157 @@ int launch_strided_copy(const void* src, int src_fp32, void* dst, int dst_fp32, 
     return B200_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Split-K reduction epilogues (conv_tc.cu launch_conv_tc_splitk): ws holds `splits` slices [P][N] of fp32 partial
+// sums; every thread adds the slices of one output vector in split order (no atomics, so the result does not depend on
+// the order in which the splits finished), then applies what the unsplit GEMM epilogue would have applied.
+// ------------------------------------------------------------------------------------------------
+
+// ConvLSTM step (the EPI_LSTM epilogue of conv_tc.cu, unet.py:29-35): the N = 4*Ch columns are gate-interleaved in
+// blocks of cht hidden channels (column (nt*4 + g)*cht + j, like bias_packed); h_next bf16, c_next fp32, no gates.
+__global__ void __launch_bounds__(256) splitk_lstm_cell_kernel(const float* __restrict__ ws, int splits, long long P,
+                                                               int Ch, int cht, const float* __restrict__ bias,
+                                                               const float* __restrict__ c_prev,
+                                                               float* __restrict__ c_next,
+                                                               __nv_bfloat16* __restrict__ h_next) {
+    constexpr int V = 8;
+    const int CV = Ch / V;
+    const long long nvec = P * CV;
+    const long long slice = P * 4LL * Ch;
+    for (long long v = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; v < nvec;
+         v += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const long long p = v / CV;
+        const int ch = static_cast<int>(v - p * CV) * V;
+        const int nt = ch / cht;
+        const int col = nt * 4 * cht + (ch - nt * cht);  // gate g at col + g * cht
+        const float* r = ws + p * 4LL * Ch + col;
+        float z[4][V];
+#pragma unroll
+        for (int g = 0; g < 4; ++g) ldv<float, V>(r + g * cht, z[g]);
+        for (int s = 1; s < splits; ++s) {
+#pragma unroll
+            for (int g = 0; g < 4; ++g) {
+                float t[V];
+                ldv<float, V>(r + s * slice + g * cht, t);
+#pragma unroll
+                for (int j = 0; j < V; ++j) z[g][j] += t[j];
+            }
+        }
+        if (bias) {
+#pragma unroll
+            for (int g = 0; g < 4; ++g) {
+                float b[V];
+                ldv<float, V>(bias + col + g * cht, b);
+#pragma unroll
+                for (int j = 0; j < V; ++j) z[g][j] += b[j];
+            }
+        }
+        float cp[V];
+        if (c_prev) {
+            ldv<float, V>(c_prev + p * Ch + ch, cp);
+        } else {
+#pragma unroll
+            for (int j = 0; j < V; ++j) cp[j] = 0.f;
+        }
+        float cn[V], hn[V];
+#pragma unroll
+        for (int j = 0; j < V; ++j) {
+            const float gi = act_sigmoid<true>(z[0][j]);
+            const float gf = act_sigmoid<true>(z[1][j]);
+            const float gg = act_tanh<true>(z[2][j]);
+            const float go = act_sigmoid<true>(z[3][j]);
+            cn[j] = fmaf(gf, cp[j], gi * gg);
+            hn[j] = go * act_tanh<true>(cn[j]);
+        }
+        stv<float, V>(c_next + p * Ch + ch, cn);
+        stv<__nv_bfloat16, V>(h_next + p * Ch + ch, hn);
+    }
+}
+
+int launch_splitk_lstm_cell(const float* ws, int splits, long long P, int Ch, int cht, const float* bias,
+                            const float* c_prev, float* c_next, void* h_next, cudaStream_t stream) {
+    if (Ch % 16 != 0 || (cht != 16 && cht != 32 && cht != 64) || Ch % cht != 0) {
+        set_last_error("splitk_lstm_cell: Ch=%d / cht=%d not supported", Ch, cht);
+        return B200_ERR_SHAPE;
+    }
+    for (const void* q : {static_cast<const void*>(ws), static_cast<const void*>(bias), static_cast<const void*>(c_prev),
+                          static_cast<const void*>(c_next), static_cast<const void*>(h_next)})
+        if (reinterpret_cast<uintptr_t>(q) & 15) {
+            set_last_error("splitk_lstm_cell: pointers must be 16-byte aligned");
+            return B200_ERR_ALIGN;
+        }
+    const long long nvec = P * (Ch / 8);
+    splitk_lstm_cell_kernel<<<grid_for(nvec, 256, num_sms() * 16), 256, 0, stream>>>(
+        ws, splits, P, Ch, cht, bias, c_prev, c_next, static_cast<__nv_bfloat16*>(h_next));
+    B200_CUDA_CHECK(cudaGetLastError());
+    return B200_OK;
+}
+
+// Convolution with eval-mode BatchNorm folded in (the EPI_STORE epilogue with scale): y = sum * scale + shift, optional
+// ReLU; scale / shift may be NULL (1 / 0).  y: bf16 or fp32 [P][N].
+template <typename TD>
+__global__ void __launch_bounds__(256) splitk_affine_kernel(const float* __restrict__ ws, int splits, long long P, int N,
+                                                            const float* __restrict__ scale,
+                                                            const float* __restrict__ shift, int relu,
+                                                            TD* __restrict__ y) {
+    constexpr int V = 8;
+    const int NV = N / V;
+    const long long nvec = P * NV;
+    const long long slice = P * static_cast<long long>(N);
+    for (long long v = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; v < nvec;
+         v += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const long long p = v / NV;
+        const int n = static_cast<int>(v - p * NV) * V;
+        const float* r = ws + p * N + n;
+        float f[V];
+        ldv<float, V>(r, f);
+        for (int s = 1; s < splits; ++s) {
+            float t[V];
+            ldv<float, V>(r + s * slice, t);
+#pragma unroll
+            for (int j = 0; j < V; ++j) f[j] += t[j];
+        }
+        if (scale) {
+            float a[V];
+            ldv<float, V>(scale + n, a);
+#pragma unroll
+            for (int j = 0; j < V; ++j) f[j] *= a[j];
+        }
+        if (shift) {
+            float b[V];
+            ldv<float, V>(shift + n, b);
+#pragma unroll
+            for (int j = 0; j < V; ++j) f[j] += b[j];
+        }
+        if (relu) {
+#pragma unroll
+            for (int j = 0; j < V; ++j) f[j] = fmaxf(f[j], 0.f);
+        }
+        stv<TD, V>(y + p * N + n, f);
+    }
+}
+
+int launch_splitk_affine(const float* ws, int splits, long long P, int N, const float* scale, const float* shift, int relu,
+                         void* y, int out_fp32, cudaStream_t stream) {
+    if (N % 16 != 0) {
+        set_last_error("splitk_affine: N=%d is not a multiple of 16", N);
+        return B200_ERR_SHAPE;
+    }
+    for (const void* q : {static_cast<const void*>(ws), static_cast<const void*>(scale), static_cast<const void*>(shift),
+                          static_cast<const void*>(y)})
+        if (reinterpret_cast<uintptr_t>(q) & 15) {
+            set_last_error("splitk_affine: pointers must be 16-byte aligned");
+            return B200_ERR_ALIGN;
+        }
+    const long long nvec = P * (N / 8);
+    const unsigned grid = grid_for(nvec, 256, num_sms() * 16);
+    if (out_fp32)
+        splitk_affine_kernel<float><<<grid, 256, 0, stream>>>(ws, splits, P, N, scale, shift, relu, static_cast<float*>(y));
+    else
+        splitk_affine_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(ws, splits, P, N, scale, shift, relu,
+                                                                     static_cast<__nv_bfloat16*>(y));
+    B200_CUDA_CHECK(cudaGetLastError());
+    return B200_OK;
+}
+
 }  // namespace b200

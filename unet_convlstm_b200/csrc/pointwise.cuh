@@ -61,6 +61,11 @@ int launch_shuffle2x2(const void* src, void* dst, const float* bias, long long I
                       int Wd, int oy, int ox, int unshuffle, int dtype_fp32, cudaStream_t stream);
 int launch_strided_copy(const void* src, int src_fp32, void* dst, int dst_fp32, const long long* dims,
                         const long long* sstr, const long long* dstr, int accumulate, cudaStream_t stream);
+// split-K reduction epilogues: ws = `splits` fp32 slices [P][N] (N = 4*Ch for the cell), added in split order
+int launch_splitk_lstm_cell(const float* ws, int splits, long long P, int Ch, int cht, const float* bias,
+                            const float* c_prev, float* c_next, void* h_next, cudaStream_t stream);
+int launch_splitk_affine(const float* ws, int splits, long long P, int N, const float* scale, const float* shift, int relu,
+                         void* y, int out_fp32, cudaStream_t stream);
 
 // ---- conv_simt.cu ----
 struct ConvSimtParams {

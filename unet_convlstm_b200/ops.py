@@ -282,16 +282,76 @@ def conv_affine_relu_ok(x0, x1, N) -> bool:
 
 def conv_affine_relu(x0, x1, wp, scale, shift, ksize, relu=True):
     """Inference: relu(conv_k([x0 ; x1]) * scale + shift) in one kernel (eval-mode BatchNorm folded into the
-    GEMM epilogue, b200_conv_affine_relu_tc_fwd).  Tensor-core path only (see conv_affine_relu_ok)."""
+    GEMM epilogue, b200_conv_affine_relu_tc_fwd).  Tensor-core path only (see conv_affine_relu_ok).  Under
+    split_k_routing(), a single frame with few M tiles is split over K instead (splitk_splits)."""
     _chk(x0, "x0"), _chk(wp, "wp")
     T, B, H, W, C0 = x0.shape
     C1 = 0 if x1 is None else _chk(x1, "x1").shape[-1]
     N = wp.shape[1]
+    splits = splitk_splits(x0, x1, N, ksize)
+    if splits > 1:
+        return conv_affine_relu_splitk(x0, x1, wp, scale, shift, ksize, splits, relu)
     out = torch.empty((T, B, H, W, N), device=x0.device, dtype=x0.dtype)
     _lib.call("b200_conv_affine_relu_tc_fwd", _p(x0), C0, _p(x1), C1, T, B, H, W, _p(wp), _p(scale), _p(shift), N, ksize,
               _p(out), int(relu), _st(), tag=f"K{C0 + C1} N{N} {H}x{W} k{ksize} +bn(eval)+relu",
               work=(2.0 * T * B * H * W * ksize * ksize * (C0 + C1) * N, None))
     return out
+
+
+# ------------------------------------------------------------------------------------------------
+# split K for single-frame problems with few M tiles (b200_splitk_splits).  Only streaming inference
+# (unet_convlstm_b200/stream.py) routes here, inside split_k_routing(); every other call keeps its kernels.
+# ------------------------------------------------------------------------------------------------
+_SPLITK_ROUTING = [False]
+
+
+class split_k_routing:
+    """`with split_k_routing():` single-frame bf16 folded convolutions (conv_affine_relu) and ConvLSTM steps
+    (lstm_seq_fwd_fused at T = 1) whose shape b200_splitk_splits selects run split over K."""
+
+    def __enter__(self):
+        self.prev, _SPLITK_ROUTING[0] = _SPLITK_ROUTING[0], True
+        return self
+
+    def __exit__(self, *exc):
+        _SPLITK_ROUTING[0] = self.prev
+        return False
+
+
+def splitk_splits(x0, x1, N, ksize) -> int:
+    """K splits for the bf16 convolution of the frame x0 [1,B,H,W,C0] (+ x1) into N channels: 1 = unsplit."""
+    if not _SPLITK_ROUTING[0] or x0.dtype != torch.bfloat16 or x0.shape[0] != 1:
+        return 1
+    _, B, H, W, C0 = x0.shape
+    C1 = 0 if x1 is None else x1.shape[-1]
+    return int(_lib.lib().b200_splitk_splits(B, H, W, C0, C1, N, ksize))
+
+
+def conv_affine_relu_splitk(x0, x1, wp, scale, shift, ksize, splits, relu=True, out_fp32=False):
+    """conv_affine_relu of one frame (x0 [1,B,H,W,C0]) split over K into `splits` ranges (b200_conv_affine_relu_splitk_tc);
+    scale / shift None: the plain convolution.  Returns [1,B,H,W,N], bf16 (fp32 with out_fp32)."""
+    _chk(x0, "x0"), _chk(wp, "wp")
+    T, B, H, W, C0 = x0.shape
+    C1 = 0 if x1 is None else _chk(x1, "x1").shape[-1]
+    N = wp.shape[1]
+    if T != 1:
+        raise ValueError(f"conv_affine_relu_splitk: one frame at a time, got T={T}")
+    out = torch.empty((1, B, H, W, N), device=x0.device, dtype=torch.float32 if out_fp32 else x0.dtype)
+    _lib.call("b200_conv_affine_relu_splitk_tc", _p(x0), C0, _p(x1), C1, B, H, W, _p(wp), _p(scale), _p(shift), N, ksize,
+              _p(out), int(out_fp32), int(relu), int(splits), _st(),
+              tag=f"K{C0 + C1} N{N} {H}x{W} k{ksize} +bn(eval)+relu splitK{splits}",
+              work=(2.0 * B * H * W * ksize * ksize * (C0 + C1) * N, None))
+    return out
+
+
+def lstm_cell_fwd_splitk(x_t, h_prev, c_prev, wp_il, bias_il, c_next, h_next, ksize, splits):
+    """One ConvLSTM step split over K (b200_convlstm_cell_fwd_splitk_tc): the fused cell without its gates output."""
+    B, H, W, Cin = x_t.shape
+    Ch = c_next.shape[-1]
+    kin = Cin + (Ch if h_prev is not None else 0)
+    _lib.call("b200_convlstm_cell_fwd_splitk_tc", _p(x_t), Cin, _p(h_prev), Ch, B, H, W, _p(wp_il), _p(bias_il),
+              _p(c_prev), _p(c_next), _p(h_next), int(splits), ksize, _st(), tag=f"Ch{Ch} {H}x{W} splitK{splits}",
+              work=(2.0 * B * H * W * ksize * ksize * kin * 4 * Ch, None))
 
 
 def bn_eval_scale_shift(gamma, beta, running_mean, running_var, eps, conv_bias):
@@ -778,6 +838,12 @@ def lstm_seq_fwd_fused(x_seq, h_all, c_all, wp_il, bias_il, gates, have_h0, ksiz
     """All T steps of one ConvLSTM layer in one timestep-persistent cooperative launch."""
     T, B, H, W, Cin = x_seq.shape
     Ch = c_all.shape[-1]
+    if T == 1:
+        splits = splitk_splits(x_seq, h_all[0] if have_h0 else None, 4 * Ch, ksize)
+        if splits > 1:   # (split_k_routing only; the gates are not written)
+            lstm_cell_fwd_splitk(x_seq[0], h_all[0] if have_h0 else None, c_all[0] if have_h0 else None, wp_il, bias_il,
+                                 c_all[1], h_all[1], ksize, splits)
+            return
     kin = Cin + Ch
     fl = 2.0 * B * H * W * ksize * ksize * 4 * Ch * (kin * T - (0 if have_h0 else Ch))
     timer = CELL_TIMER
