@@ -121,7 +121,7 @@ int b200_conv_tf32_supported(int B, int H, int W, int C0, int C1, int N, int lst
 int b200_conv_tf32_fwd(const float* src0, int C0, const float* src1, int C1, int T, int B, int H, int W,
                        const float* wpacked, const float* bias, int N, int ksize, float* dst0, long long ld0, int split,
                        float* dst1, long long ld1, int relu, int accumulate, void* stream);
-/* Weight gradient in the tf32 mode; arguments as b200_wgrad_tc with fp32 dz / src (dw zero-initialised by the caller). */
+/* Weight gradient in the tf32 mode: dw += ..., arguments and reduction as b200_wgrad_tc with fp32 dz / src. */
 int b200_wgrad_tf32_supported(int B, int H, int W, int Nz, int Csrc);
 int b200_wgrad_tf32(const float* dz, int Nz, const float* src, int Csrc, int T, int B, int H, int W, int ksize, float* dw,
                     long long ldk, int koff, void* stream);
@@ -157,10 +157,16 @@ int b200_convlstm_seq_bwd_tc(void* dz_all, const void* wd_packed, const void* ga
 /* Weight gradient of a convolution, summed over all T*B images (autograd of nn.Conv2d, unet.py:19
  * and :70-71; for the ConvLSTM this is the BPTT sum over timesteps):
  *   dw[tap][n][koff + k] += sum_{t,p} dz[t,p,n] * src[t, p+tap, k]
- * dz: bf16 [T][B][H][W][Nz], src: bf16 [T][B][H][W][Csrc], dw: fp32 [k*k][Nz][ldk], zero-initialised
- * by the caller (partial sums are combined with fp32 reductions). */
+ * dz: bf16 [T][B][H][W][Nz], src: bf16 [T][B][H][W][Csrc], dw: fp32 [k*k][Nz][ldk]; columns outside
+ * [koff, koff + Csrc) are not touched.  The reduction over t,p is split; each split stores its partial sums to its own
+ * slice of the per-stream workspace and a second kernel adds the slices to dw in split order, at any split count
+ * (one included): the result does not depend on which split finishes first. */
 int b200_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
                   int ksize, float* dw, long long ldk, int koff, void* stream);
+/* The kernel b200_wgrad_tc (in_fp32 = 0) or b200_wgrad_tf32 (in_fp32 = 1) runs for this problem and its number of
+ * reduction splits, without launching anything: plan[0] = 0 wgrad_tc, 1 wgrad_tc2, 2 wgrad_halo; plan[1] = splits. */
+int b200_wgrad_plan(int Nz, int Csrc, int T, int B, int H, int W, int ksize, long long ldk, int koff, int in_fp32,
+                    int* plan);
 
 /* 1 if b200_wgrad_tc can tile this problem. */
 int b200_wgrad_tc_supported(int B, int H, int W, int Nz, int Csrc);

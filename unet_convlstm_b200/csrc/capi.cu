@@ -10,16 +10,20 @@
 using namespace b200;
 
 namespace b200 {
+// *_splits: the reduction splits the launch of that shape uses (negative: an error code)
 int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
                     int ksize, float* dw, long long ldk, int koff, cudaStream_t stream, int in_fp32 = 0);
+int wgrad_tc_splits(int Nz, int Csrc, int T, int B, int H, int W, int ksize, int in_fp32);
 // wgrad_halo.cu: 64-channel 3x3 layers, source tile loaded once per pixel block
 bool wgrad_halo_supported(int Nz, int Csrc, int B, int H, int W, int ksize);
 int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, float* dw,
                       long long ldk, int koff, cudaStream_t stream);
+int wgrad_halo_splits(int Nz, int Csrc, int T, int B, int H, int W);
 // wgrad_tc2.cu: narrow sources on a CTA pair (tcgen05 cta_group::2)
 bool wgrad_tc2_supported(int Nz, int Csrc, int ksize);
 int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, int ksize, float* dw,
                      long long ldk, int koff, cudaStream_t stream);
+int wgrad_tc2_splits(int Nz, int Csrc, int T, int B, int H, int W, int ksize);
 }
 
 extern "C" int b200_device_error(void) {
@@ -391,12 +395,10 @@ extern "C" int b200_convlstm_seq_bwd_tc(void* dz_all, const void* wd_packed, con
     return launch_convlstm_seq_bwd_tc(wd_packed, p, static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int b200_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
-                             int ksize, float* dw, long long ldk, int koff, void* stream) {
-    if (!dz || !src || !dw || Nz <= 0 || Csrc <= 0 || (ksize & 1) == 0 || koff < 0 || koff + Csrc > ldk) {
-        set_last_error("b200_wgrad_tc: bad arguments");
-        return B200_ERR_ARG;
-    }
+enum { WGRAD_KERNEL_TC = 0, WGRAD_KERNEL_TC2 = 1, WGRAD_KERNEL_HALO = 2 };
+
+// the kernel b200_wgrad_tc runs for this problem
+static int wgrad_kernel(int Nz, int Csrc, int B, int H, int W, int ksize, long long ldk, int koff) {
     // B200_WGRAD_HALO (default 1): the halo kernel (wgrad_halo.cu) for the 64-channel 3x3 layers -- source tile
     // loaded once per pixel block, taps as shifted MN-major descriptors: 820 -> 1090 TFLOP/s at Nz = 64, 64x64
     static const int halo_mode = [] {
@@ -404,7 +406,7 @@ extern "C" int b200_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, 
         return e ? atoi(e) : 1;
     }();
     if (halo_mode > 0 && (ldk % 4) == 0 && (koff % 4) == 0 && wgrad_halo_supported(Nz, Csrc, B, H, W, ksize))
-        return launch_wgrad_halo(dz, Nz, src, Csrc, T, B, H, W, dw, ldk, koff, static_cast<cudaStream_t>(stream));
+        return WGRAD_KERNEL_HALO;
     // B200_WGRAD_2CTA: the CTA-pair kernel (wgrad_tc2.cu).  0 = never, 1 (default) = where it measured faster or
     // equal (profiles/r01_wgrad_2cta_ab.txt): every wide-source shape it supports (1.00-1.19x) and 64-channel sources
     // with dz >= 128 channels (912 -> 1100 TFLOP/s; at Nz = 64 both kernels sit at the L2 -> SM fill limit of the
@@ -415,9 +417,41 @@ extern "C" int b200_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, 
     }();
     if (pair_mode > 0 && (pair_mode >= 2 || Csrc > 64 || (Csrc == 64 && Nz >= 128)) && (ldk % 4) == 0 && (koff % 4) == 0 &&
         wgrad_tc2_supported(Nz, Csrc, ksize))
-        return launch_wgrad_tc2(dz, Nz, src, Csrc, T, B, H, W, ksize, dw, ldk, koff, static_cast<cudaStream_t>(stream));
-    return launch_wgrad_tc(dz, Nz, src, Csrc, T, B, H, W, ksize, dw, ldk, koff,
-                           static_cast<cudaStream_t>(stream));
+        return WGRAD_KERNEL_TC2;
+    return WGRAD_KERNEL_TC;
+}
+
+extern "C" int b200_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
+                             int ksize, float* dw, long long ldk, int koff, void* stream) {
+    if (!dz || !src || !dw || Nz <= 0 || Csrc <= 0 || (ksize & 1) == 0 || koff < 0 || koff + Csrc > ldk) {
+        set_last_error("b200_wgrad_tc: bad arguments");
+        return B200_ERR_ARG;
+    }
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (wgrad_kernel(Nz, Csrc, B, H, W, ksize, ldk, koff)) {
+        case WGRAD_KERNEL_HALO: return launch_wgrad_halo(dz, Nz, src, Csrc, T, B, H, W, dw, ldk, koff, st);
+        case WGRAD_KERNEL_TC2: return launch_wgrad_tc2(dz, Nz, src, Csrc, T, B, H, W, ksize, dw, ldk, koff, st);
+        default: return launch_wgrad_tc(dz, Nz, src, Csrc, T, B, H, W, ksize, dw, ldk, koff, st);
+    }
+}
+
+extern "C" int b200_wgrad_plan(int Nz, int Csrc, int T, int B, int H, int W, int ksize, long long ldk, int koff,
+                               int in_fp32, int* plan) {
+    if (!plan || Nz <= 0 || Csrc <= 0 || T <= 0 || (ksize & 1) == 0 || koff < 0 || koff + Csrc > ldk) {
+        set_last_error("b200_wgrad_plan: bad arguments");
+        return B200_ERR_ARG;
+    }
+    const int kernel = in_fp32 ? WGRAD_KERNEL_TC : wgrad_kernel(Nz, Csrc, B, H, W, ksize, ldk, koff);
+    int splits;
+    switch (kernel) {
+        case WGRAD_KERNEL_HALO: splits = wgrad_halo_splits(Nz, Csrc, T, B, H, W); break;
+        case WGRAD_KERNEL_TC2: splits = wgrad_tc2_splits(Nz, Csrc, T, B, H, W, ksize); break;
+        default: splits = wgrad_tc_splits(Nz, Csrc, T, B, H, W, ksize, in_fp32); break;
+    }
+    if (splits < 0) return splits;
+    plan[0] = kernel;
+    plan[1] = splits;
+    return B200_OK;
 }
 
 // "tf32" precision mode: the weight gradient from fp32 dz / src on tcgen05 kind::tf32 (MN-major operands, 32 pixels per

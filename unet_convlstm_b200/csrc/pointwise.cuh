@@ -87,7 +87,7 @@ int launch_conv_simt(const ConvSimtParams& p, int dtype_fp32, cudaStream_t strea
 struct WgradSimtParams {
     const void* dz;
     const void* src;
-    float* dw;          // [taps][Nz][ldk], accumulated into (caller zero-fills)
+    float* dw;          // [taps][Nz][ldk], accumulated into
     int IMG, H, W;
     int Nz, Csrc, ksize, pad;
     long long ldk;

@@ -43,7 +43,7 @@ struct WgradHaloParams {
     int s_tiles;       // Nz / 64
     uint32_t src_bytes, src_stage_bytes;
     int stages;        // pipeline depth that fits in shared memory (3 or 4)
-    float* dw;         // with splits > 1 the split-K workspace, split s at dw + s * split_stride
+    float* dw;         // the split-K workspace, split s at dw + s * split_stride
     long long ldk;
     int koff;
     long long split_stride;
@@ -247,13 +247,14 @@ bool wgrad_halo_supported(int Nz, int Csrc, int B, int H, int W, int ksize) {
     return H % Ht == 0 && B > 0;
 }
 
-int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, float* dw,
-                      long long ldk, int koff, cudaStream_t stream) {
+// Tiling and reduction split of a launch: every field of p except the pointers, the output layout and the stages.
+static int plan_wgrad_halo(int Nz, int Csrc, int T, int B, int H, int W, WgradHaloParams* pp) {
     if (!wgrad_halo_supported(Nz, Csrc, B, H, W, 3)) {
         set_last_error("wgrad_halo: shape not supported");
         return B200_ERR_SHAPE;
     }
-    WgradHaloParams p = {};
+    WgradHaloParams& p = *pp;
+    p = {};
     p.T = T; p.B = B; p.H = H; p.W = W; p.Nz = Nz; p.Cs = Csrc;
     p.Ht = WH_RB / W;
     p.P = W + 2;
@@ -278,21 +279,34 @@ int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, 
     }
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
-    p.dw = dw; p.ldk = ldk; p.koff = koff;
-    if (p.splits > 1) {
-        p.split_stride = 9LL * Nz * Csrc;
-        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
-        if (!p.dw) {
-            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
-            return B200_ERR_CUDA;
-        }
-        p.ldk = Csrc;
-        p.koff = 0;
+    return B200_OK;
+}
+
+int wgrad_halo_splits(int Nz, int Csrc, int T, int B, int H, int W) {
+    WgradHaloParams p;
+    const int rc = plan_wgrad_halo(Nz, Csrc, T, B, H, W, &p);
+    return rc == B200_OK ? p.splits : rc;
+}
+
+// dw += the weight gradient, at any split count (see launch_wgrad_tc)
+int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, float* dw,
+                      long long ldk, int koff, cudaStream_t stream) {
+    WgradHaloParams p;
+    int rc = plan_wgrad_halo(Nz, Csrc, T, B, H, W, &p);
+    if (rc != B200_OK) return rc;
+    const int nsm = num_sms();
+    p.split_stride = 9LL * Nz * Csrc;
+    p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+    if (!p.dw) {
+        set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+        return B200_ERR_CUDA;
     }
+    p.ldk = Csrc;
+    p.koff = 0;
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
-    int rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, 64, W, p.Ht, 1);
+    rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, 64, W, p.Ht, 1);
     if (rc != B200_OK) return rc;
     rc = make_act_tmap(&ts, src, Csrc, W, H, B, T, Csrc, p.P, p.Ht + 2, 1);
     if (rc != B200_OK) return rc;
@@ -317,7 +331,6 @@ int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, 
     const int grid = total < nsm ? total : nsm;
     wgrad_halo_kernel<<<grid, WH_THREADS, smem, stream>>>(tz, ts, p);
     B200_CUDA_CHECK(cudaGetLastError());
-    if (p.splits == 1) return B200_OK;
     return splitk_reduce(p.dw, p.splits, 9LL * Nz, Csrc, dw, ldk, koff, stream);
 }
 

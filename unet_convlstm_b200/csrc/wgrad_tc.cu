@@ -25,9 +25,9 @@
 //     128 dz channels would be half empty, so the roles are swapped: A = G = 128/Csrc tap-shifted
 //     source boxes stacked along M (rows = (tap, source channel)), B = dz channels (N).
 //
-// Work units = (reduction split) x (tap-group set, S tile, V tile); with more than one split each split stores its
+// Work units = (reduction split) x (tap-group set, S tile, V tile); every split, a single one too, stores its
 // partial sums to its own workspace slice and splitk_reduce (common.cu) adds them to dw in split order, so the
-// result is the same from run to run.
+// result is the same from run to run and is added to dw at any split count.
 // Warp roles: warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue.
 #include "common.cuh"
 #include "ptx.cuh"
@@ -52,7 +52,7 @@ struct WgradParams {
     int GU;          // groups (accumulators) per unit
     int ngsets;      // ceil(ngroups / GU)
     int s_tiles, v_tiles, out_tiles;
-    float* dw;       // [taps][Nz][ldk]; with splits > 1 the split-K workspace, split s at dw + s * split_stride
+    float* dw;       // the split-K workspace, split s at dw + s * split_stride: [taps][Nz][ldk = Csrc], koff = 0
     long long ldk;
     int koff;
     long long split_stride;
@@ -450,13 +450,14 @@ static int chunk_width(int C, int esize) {
     return 0;
 }
 
-// dw must be zero-initialised by the caller (partial sums of the reduction splits are added to it).
-// in_fp32: dz / src are fp32 tensors and the products are TF32 (see WgradParams::in_fp32).
-int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
-                    int ksize, float* dw, long long ldk, int koff, cudaStream_t stream, int in_fp32) {
+// Tiling and reduction split of a launch: every field of p except the pointers and the output layout.
+static int plan_wgrad_tc(int Nz, int Csrc, int T, int B, int H, int W, int ksize, int in_fp32, WgradParams* pp,
+                         MTile* pmt, bool* pstacked, int* pblock_n) {
     const int esize = in_fp32 ? 4 : 2;
     const int rb_pixels = 128 / esize;   // pixels per pipeline stage: 64 (bf16) or 32 (fp32)
-    WgradParams p = {};
+    WgradParams& p = *pp;
+    MTile& mt = *pmt;
+    p = {};
     p.in_fp32 = in_fp32;
     p.T = T; p.B = B; p.H = H; p.W = W;
     p.Nz = Nz; p.Csrc = Csrc; p.ksize = ksize; p.pad = ksize / 2; p.taps = ksize * ksize;
@@ -467,11 +468,6 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
         set_last_error("wgrad_tc: channels Nz=%d Csrc=%d not multiples of %d", Nz, Csrc, 32 / esize);
         return B200_ERR_SHAPE;
     }
-    if ((ldk % 4) != 0 || (koff % 4) != 0) {
-        set_last_error("wgrad_tc: ldk/koff must be multiples of 4");
-        return B200_ERR_ALIGN;
-    }
-    MTile mt;
     if (!plan_mtile(B, H, W, rb_pixels, &mt)) {
         set_last_error("wgrad_tc: spatial shape B=%d H=%d W=%d cannot be tiled", B, H, W);
         return B200_ERR_SHAPE;
@@ -482,7 +478,8 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
     // few source channels: stack G taps of the source along M, dz becomes the N operand
     // (the stacked source box is ONE channel chunk: its pixel row must fit the 128-byte swizzle span)
     const bool stacked = (Csrc * esize == 32 || Csrc * esize == 64 || Csrc * esize == 128) && p.taps > 1;
-    int block_n;
+    int& block_n = *pblock_n;
+    *pstacked = stacked;
     if (stacked) {
         p.G = WG_BLOCK_M / Csrc;
         p.cwV = Csrc;
@@ -520,21 +517,46 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
     }
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
-    p.dw = dw; p.ldk = ldk; p.koff = koff;
-    if (p.splits > 1) {
-        p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
-        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
-        if (!p.dw) {
-            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
-            return B200_ERR_CUDA;
-        }
-        p.ldk = Csrc;
-        p.koff = 0;
+    return B200_OK;
+}
+
+int wgrad_tc_splits(int Nz, int Csrc, int T, int B, int H, int W, int ksize, int in_fp32) {
+    WgradParams p;
+    MTile mt;
+    bool stacked;
+    int block_n;
+    const int rc = plan_wgrad_tc(Nz, Csrc, T, B, H, W, ksize, in_fp32, &p, &mt, &stacked, &block_n);
+    return rc == B200_OK ? p.splits : rc;
+}
+
+// dw += the weight gradient, at any split count: every split stores its partial sums to its own workspace slice and
+// splitk_reduce adds the slices to dw.  in_fp32: dz / src are fp32 tensors and the products are TF32 (see
+// WgradParams::in_fp32).
+int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W,
+                    int ksize, float* dw, long long ldk, int koff, cudaStream_t stream, int in_fp32) {
+    const int esize = in_fp32 ? 4 : 2;
+    if ((ldk % 4) != 0 || (koff % 4) != 0) {
+        set_last_error("wgrad_tc: ldk/koff must be multiples of 4");
+        return B200_ERR_ALIGN;
     }
+    WgradParams p;
+    MTile mt;
+    bool stacked;
+    int block_n;
+    int rc = plan_wgrad_tc(Nz, Csrc, T, B, H, W, ksize, in_fp32, &p, &mt, &stacked, &block_n);
+    if (rc != B200_OK) return rc;
+    p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
+    p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+    if (!p.dw) {
+        set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+        return B200_ERR_CUDA;
+    }
+    p.ldk = Csrc;
+    p.koff = 0;
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
-    int rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, p.cwS, mt.Wt, mt.Ht, mt.Bt, esize, in_fp32);
+    rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, p.cwS, mt.Wt, mt.Ht, mt.Bt, esize, in_fp32);
     if (rc != B200_OK) return rc;
     rc = make_act_tmap(&ts, src, Csrc, W, H, B, T, p.cwV, mt.Wt, mt.Ht, mt.Bt, esize, in_fp32);
     if (rc != B200_OK) return rc;
@@ -551,7 +573,7 @@ int launch_wgrad_tc(const void* dz, int Nz, const void* src, int Csrc, int T, in
             default: rc = launch_wgrad_impl<64, false>(tz, ts, p, stream); break;
         }
     }
-    if (rc != B200_OK || p.splits == 1) return rc;
+    if (rc != B200_OK) return rc;
     return splitk_reduce(p.dw, p.splits, static_cast<long long>(p.taps) * Nz, Csrc, dw, ldk, koff, stream);
 }
 

@@ -45,7 +45,7 @@ struct Wgrad2Params {
     int ngroups, GU, ngsets;
     int gset_inner;             // unit order: tap sets fastest (1) or slowest (0)
     int s_tiles, v_tiles, out_tiles;
-    float* dw;                  // with splits > 1 the split-K workspace, split s at dw + s * split_stride
+    float* dw;                  // the split-K workspace, split s at dw + s * split_stride
     long long ldk;
     int koff;
     long long split_stride;
@@ -429,14 +429,16 @@ bool wgrad_tc2_supported(int Nz, int Csrc, int ksize) {
     return Csrc % block_n == 0;
 }
 
-int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, int ksize, float* dw,
-                     long long ldk, int koff, cudaStream_t stream) {
-    Wgrad2Params p = {};
+// Tiling and reduction split of a launch: every field of p except the pointers and the output layout.
+static int plan_wgrad_tc2(int Nz, int Csrc, int T, int B, int H, int W, int ksize, Wgrad2Params* pp, MTile* pmt,
+                          int* pblock_n) {
+    Wgrad2Params& p = *pp;
+    MTile& mt = *pmt;
+    int& block_n = *pblock_n;
+    p = {};
     p.T = T; p.B = B; p.H = H; p.W = W;
     p.Nz = Nz; p.Csrc = Csrc; p.ksize = ksize; p.pad = ksize / 2; p.taps = ksize * ksize;
     const bool stacked = w2_stacked(Csrc, ksize);
-    int block_n;
-    MTile mt;
     if (!plan_mtile(B, H, W, W2_RB, &mt)) {
         set_last_error("wgrad_tc2: spatial shape B=%d H=%d W=%d cannot be tiled", B, H, W);
         return B200_ERR_SHAPE;
@@ -487,21 +489,38 @@ int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, i
     }
     p.rb_per_split = (p.num_rblocks + best - 1) / best;
     p.splits = (p.num_rblocks + p.rb_per_split - 1) / p.rb_per_split;
-    p.dw = dw; p.ldk = ldk; p.koff = koff;
-    if (p.splits > 1) {
-        p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
-        p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
-        if (!p.dw) {
-            set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
-            return B200_ERR_CUDA;
-        }
-        p.ldk = Csrc;
-        p.koff = 0;
+    return B200_OK;
+}
+
+int wgrad_tc2_splits(int Nz, int Csrc, int T, int B, int H, int W, int ksize) {
+    Wgrad2Params p;
+    MTile mt;
+    int block_n;
+    const int rc = plan_wgrad_tc2(Nz, Csrc, T, B, H, W, ksize, &p, &mt, &block_n);
+    return rc == B200_OK ? p.splits : rc;
+}
+
+// dw += the weight gradient, at any split count (see launch_wgrad_tc)
+int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, int B, int H, int W, int ksize, float* dw,
+                     long long ldk, int koff, cudaStream_t stream) {
+    Wgrad2Params p;
+    MTile mt;
+    int block_n;
+    int rc = plan_wgrad_tc2(Nz, Csrc, T, B, H, W, ksize, &p, &mt, &block_n);
+    if (rc != B200_OK) return rc;
+    const bool stacked = w2_stacked(Csrc, ksize);
+    p.split_stride = static_cast<long long>(p.taps) * Nz * Csrc;
+    p.dw = splitk_workspace(stream, static_cast<size_t>(p.splits) * p.split_stride);
+    if (!p.dw) {
+        set_last_error("%s: no split-K workspace (cudaMalloc failed, or growth during graph capture)", __func__);
+        return B200_ERR_CUDA;
     }
+    p.ldk = Csrc;
+    p.koff = 0;
     p.err_flag = device_error_flag();
 
     CUtensorMap tz, ts;
-    int rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, p.cwS, mt.Wt, mt.Ht, mt.Bt);
+    rc = make_act_tmap(&tz, dz, Nz, W, H, B, T, p.cwS, mt.Wt, mt.Ht, mt.Bt);
     if (rc != B200_OK) return rc;
     rc = make_act_tmap(&ts, src, Csrc, W, H, B, T, p.cwV, mt.Wt, mt.Ht, mt.Bt);
     if (rc != B200_OK) return rc;
@@ -518,7 +537,7 @@ int launch_wgrad_tc2(const void* dz, int Nz, const void* src, int Csrc, int T, i
             default: rc = launch_wgrad2_impl<64, false>(tz, ts, p, stream); break;
         }
     }
-    if (rc != B200_OK || p.splits == 1) return rc;
+    if (rc != B200_OK) return rc;
     return splitk_reduce(p.dw, p.splits, static_cast<long long>(p.taps) * Nz, Csrc, dw, ldk, koff, stream);
 }
 

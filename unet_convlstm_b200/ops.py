@@ -368,7 +368,7 @@ def bn_eval_scale_shift(gamma, beta, running_mean, running_var, eps, conv_bias):
 
 
 def conv_wgrad(dz, src, ksize, dw, koff):
-    """dw[tap][n][koff + c] += sum_{t,p} dz[t,p,n] * src[t,p+tap,c]; dw fp32 [k*k, Nz, ldk] (pre-zeroed)."""
+    """dw[tap][n][koff + c] += sum_{t,p} dz[t,p,n] * src[t,p+tap,c]; dw fp32 [k*k, Nz, ldk]."""
     _chk(dz, "dz"), _chk(src, "src"), _chk(dw, "dw")
     T, B, H, W, Nz = dz.shape
     Cs = src.shape[-1]
