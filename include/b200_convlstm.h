@@ -307,6 +307,22 @@ int b200_wl1_grad_loss_bwd(const float* y_pred, const float* y, const float* mas
 int b200_denorm_metrics_accum(const float* y_pred, const float* y, const float* mask, long long n, int transform,
                               double trans_min, double trans_max, double y_scale, double* acc, void* stream);
 
+/* One training batch of the reference's NPZSequenceDataset (unet.py:393-401 + default_collate) from the raw dataset
+ * kept in device memory, in one launch: for b < B, row n = idx[b] (idx: int64 [B] on the device),
+ *   mask[b,t,0] = X[n,t,0] > 1.1f;  x[b,t,c] = X[n,t,c] / (float)norm_const (IEEE fp32 division);
+ *   y[b,t,0]    = 2 * (tr(clip(Y[n,t,0])) - trans_min) / trans_range - 1, rounded once to fp32,
+ * where clip (if clip != 0) bounds by [min_vel, max_vel] like np.clip, tr is transform 0 = identity, 1 = asinh(v /
+ * y_scale), 2 = sign(v) * log1p(|v| / y_scale), and trans_range = trans_max - trans_min as the caller computed it.
+ * The dtypes follow NumPy: fp64_transform = 1 runs clip, transform and affine map in fp64 (np.float64 clip bounds),
+ * fp64_affine = 1 only the affine map (np.float64 trans_min); otherwise every step is fp32 with the constants rounded to
+ * fp32.  X: fp32 [N][T][Cx][H][W], Y: fp32 [N][T][1][H][W]; x: fp32 [B][T][Cx][H][W], y / mask: fp32 [B][T][1][H][W],
+ * all contiguous.  16-byte accesses when H*W % 4 == 0 and the bases are 16-byte aligned, scalar ones otherwise.  An idx
+ * outside [0, N) is never read: its item comes out as x = y = NaN, mask = 0 (callers check indices beforehand). */
+int b200_sequence_batch(const float* X, const float* Y, long long N, int T, int Cx, int H, int W, const void* idx, int B,
+                        double norm_const, int clip, double min_vel, double max_vel, int transform, double y_scale,
+                        double trans_min, double trans_range, int fp64_transform, int fp64_affine, float* x, float* y,
+                        float* mask, void* stream);
+
 /* Gradient clipping + AdamW of the reference's step (main.py:106 clip_grad_norm_(params, 1.0); main.py:275
  * torch.optim.AdamW) over a LIST of fp32 tensors.  The pointer arrays (params, grads, ...) and numel live in HOST
  * memory and hold n device pointers / element counts; they are copied into the kernel parameters (48 tensors per

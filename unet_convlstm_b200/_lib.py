@@ -60,7 +60,7 @@ KERNELS_PER_CALL = {
     "b200_maxpool2_fwd": 1, "b200_maxpool2_bwd": 1, "b200_bn_relu_apply_pool": 1, "b200_bn_relu_pool_bwd_reduce": 1,
     "b200_bn_relu_pool_bwd_apply": 1, "b200_bn_relu_outconv_fwd": 1, "b200_bn_relu_outconv_bwd_reduce": 2,
     "b200_bn_relu_outconv_bwd_apply": 1, "b200_lstm_gates_fwd": 1, "b200_lstm_gates_bwd": 1,
-    "b200_colsum": 2, "b200_wl1_grad_loss_fwd": 2, "b200_wl1_grad_loss_bwd": 1, "b200_denorm_metrics_accum": 1, "b200_pack_weight": 1, "b200_unpack_wgrad": 1, "b200_grad_sqnorm_multi": 1, "b200_grad_clip_multi": 1, "b200_adamw_multi": 1, "b200_adamw_pack": 1, "b200_adamw_pack_multi": 1, "b200_outconv_fwd": 1, "b200_outconv_bwd": 5, "b200_shuffle2x2": 1, "b200_strided_copy": 1,
+    "b200_colsum": 2, "b200_wl1_grad_loss_fwd": 2, "b200_wl1_grad_loss_bwd": 1, "b200_denorm_metrics_accum": 1, "b200_sequence_batch": 1, "b200_pack_weight": 1, "b200_unpack_wgrad": 1, "b200_grad_sqnorm_multi": 1, "b200_grad_clip_multi": 1, "b200_adamw_multi": 1, "b200_adamw_pack": 1, "b200_adamw_pack_multi": 1, "b200_outconv_fwd": 1, "b200_outconv_bwd": 5, "b200_shuffle2x2": 1, "b200_strided_copy": 1,
 }
 
 

@@ -311,13 +311,22 @@ int launch_wgrad_halo(const void* dz, int Nz, const void* src, int Csrc, int T, 
     rc = make_act_tmap(&ts, src, Csrc, W, H, B, T, Csrc, p.P, p.Ht + 2, 1);
     if (rc != B200_OK) return rc;
     const int stage_bytes = static_cast<int>(p.src_stage_bytes + WH_DZ_BYTES);
-    p.stages = (227 * 1024 - 1280) / stage_bytes;
+    // The MMAs read source-tile rows past the loaded box: the unused second tap of the (2,2) pair (64 channels), and
+    // slots 3..7 of the M operand, which sit 3P..7P rows after the taps (16 channels).  Those rows are never stored,
+    // but they must lie inside the shared-memory allocation.  From a stage other than the last they fall into the next
+    // stage; the last stage needs `tail` bytes after it, which also hold the barriers (256 bytes).  The 16-channel
+    // first layer at W = 128 (P = 130, one image row per block) reads 3.5 KB past its stage: without this tail the
+    // last stage read past the end of shared memory and the launch stopped with an illegal-address error.
+    const int row0_max = (p.Ht - 1) * p.P + W - 16;  // tile row of tap (0, 0) in the last K step of a block
+    const int read_end = (Csrc == 64 ? row0_max + 2 * p.P + 2 + 1 + 16 : row0_max + 2 + 7 * p.P + 16) * Csrc * 2;
+    const int tail = read_end - stage_bytes > 256 ? read_end - stage_bytes : 256;
+    p.stages = (227 * 1024 - 1024 - tail) / stage_bytes;
     if (p.stages > WH_STAGES) p.stages = WH_STAGES;
     if (p.stages < 2) {
         set_last_error("wgrad_halo: tile does not fit in shared memory");
         return B200_ERR_SHAPE;
     }
-    const int smem = p.stages * stage_bytes + 1024 + 256;
+    const int smem = p.stages * stage_bytes + 1024 + tail;
     static PerDeviceOnce attr_once;  // kernel attributes are per device
     if (attr_once.first()) {
         B200_CUDA_CHECK(cudaFuncSetAttribute(wgrad_halo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));

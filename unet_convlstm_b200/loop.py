@@ -21,7 +21,7 @@ import math
 import torch
 
 from . import _lib
-from .data import DevicePrefetcher
+from .data import DeviceLoader, DevicePrefetcher, DeviceSequenceData
 from .loss import compute_loss
 from .optim import AdamW
 from .ops import _p, _st
@@ -99,13 +99,17 @@ def _device_batches(loader, device):
         cur, staged = nxt_dev, nxt_staged
 
 
-def make_loaders(dataset, batch_size, seed=42, train_fraction=0.8, rank=None, world=None):
+def make_loaders(dataset, batch_size, seed=42, train_fraction=0.8, rank=None, world=None, device=None):
     """The data pipeline of main.py:241-246 for one rank of a data-parallel job: the same 80/20 random split on every
     rank (seeded -- main.py splits unseeded, a single process does not care), then a per-rank DistributedSampler over
     the training part (shuffled, re-seeded per epoch by `loader.sampler.set_epoch(e)`) and over the validation part
-    (in order).  `batch_size` is per rank.  With world == 1 this is exactly main.py's pair of DataLoaders."""
+    (in order).  `batch_size` is per rank.  With world == 1 this is exactly main.py's pair of DataLoaders.
+
+    device: None returns those host DataLoaders.  A CUDA device uploads the dataset once (data.DeviceSequenceData) and
+    returns a pair of data.DeviceLoader with the same split, samplers and seeds: the same batches in the same order,
+    each built on the device by one kernel launch instead of NPZSequenceDataset.__getitem__ on the host."""
     import torch.distributed as dist
-    from torch.utils.data import DataLoader, DistributedSampler, random_split
+    from torch.utils.data import DataLoader, DistributedSampler, RandomSampler, SequentialSampler, random_split
     if world is None:
         world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     if rank is None:
@@ -115,12 +119,22 @@ def make_loaders(dataset, batch_size, seed=42, train_fraction=0.8, rank=None, wo
     train_ds, val_ds = random_split(dataset, [n_train, len(dataset) - n_train], generator=gen)
     if world == 1:
         g2 = torch.Generator().manual_seed(seed)
-        return (DataLoader(train_ds, batch_size=batch_size, shuffle=True, pin_memory=True, generator=g2),
-                DataLoader(val_ds, batch_size=batch_size, shuffle=False, pin_memory=True))
-    ts = DistributedSampler(train_ds, num_replicas=world, rank=rank, shuffle=True, seed=seed, drop_last=False)
-    vs = DistributedSampler(val_ds, num_replicas=world, rank=rank, shuffle=False, drop_last=False)
-    return (DataLoader(train_ds, batch_size=batch_size, sampler=ts, pin_memory=True),
-            DataLoader(val_ds, batch_size=batch_size, sampler=vs, pin_memory=True))
+        if device is None:
+            return (DataLoader(train_ds, batch_size=batch_size, shuffle=True, pin_memory=True, generator=g2),
+                    DataLoader(val_ds, batch_size=batch_size, shuffle=False, pin_memory=True))
+        ts, vs, tgen = RandomSampler(train_ds, generator=g2), SequentialSampler(val_ds), g2
+    else:
+        ts = DistributedSampler(train_ds, num_replicas=world, rank=rank, shuffle=True, seed=seed, drop_last=False)
+        vs = DistributedSampler(val_ds, num_replicas=world, rank=rank, shuffle=False, drop_last=False)
+        if device is None:
+            return (DataLoader(train_ds, batch_size=batch_size, sampler=ts, pin_memory=True),
+                    DataLoader(val_ds, batch_size=batch_size, sampler=vs, pin_memory=True))
+        tgen = None
+    data = DeviceSequenceData(dataset, device)
+    # DataLoader(shuffle=True, generator=g2) draws its base seed from g2; the other loaders draw it from torch's
+    # default generator, and so do these
+    return (DeviceLoader(data, ts, batch_size, rows=train_ds.indices, generator=tgen),
+            DeviceLoader(data, vs, batch_size, rows=val_ds.indices))
 
 
 def _stack(output):
