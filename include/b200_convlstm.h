@@ -265,6 +265,25 @@ int b200_outconv_fwd(const void* x, const float* w, const float* b, float* y, lo
 int b200_outconv_bwd(const void* x, const float* w, const float* dy, long long P, int C, int O, int dtype_fp32,
                      void* dx, double* workspace, float* dw, float* db, int accumulate, void* stream);
 
+/* SpatialAttention (unet.py:113-125; TemporalUNetDualView(use_attention=True) applies it to the bottleneck output):
+ *   y = x * a,  a = sigmoid(conv_k([mean_c x ; amax_c x]))   (2 -> 1 channels, padding k/2, no bias; k = 1, 3, 5 or 7)
+ * per image of x [IMG][H][W][C] (bf16, or fp32 if dtype_fp32; y and dx alike).  w: fp32 [2][k][k] (nn.Conv2d weight
+ * [1, 2, k, k]), read from device memory at run time.  Forward writes pooled fp32 [IMG][H][W][2] (mean, max) and a fp32
+ * [IMG][H][W], both inputs of the backward.  Backward, given dy: with ds = (sum_c dy*x) * (1-a) * a and (dmean, dmax) the
+ * transposed convolution of ds,
+ *   dx = dy*a + dmean / C + [x == max] * dmax / (number of channels equal to the max)     (dx may be NULL: not computed)
+ *   dw = sum over pixels of ds * pooled at the tap's pixel                               (dw may be NULL: not computed)
+ * the max split evenly among ties as torch.amax's backward does.  ws: fp32 workspace of 2*P + ceil(P / 2048) * 2*k*k
+ * floats, P = IMG*H*W; dw is summed per range of 2048 pixels and the ranges added in order: no atomics, run-to-run
+ * bit-identical.  16-byte accesses when C * element size is a multiple of 16 and the activation pointers are 16-byte
+ * aligned, scalar ones otherwise.  pooled must be 8-byte aligned (the backward reads it as float2; B200_ERR_ALIGN
+ * otherwise).  Kernel launches: 2 forward; backward 2, +1 with dx, +2 with dw (the sums and splitk_reduce). */
+int b200_spatial_attention_fwd(const void* x, const float* w, long long IMG, int H, int W, int C, int ksize,
+                               int dtype_fp32, float* pooled, float* a, void* y, void* stream);
+int b200_spatial_attention_bwd(const void* x, const void* dy, const float* w, const float* pooled, const float* a,
+                               long long IMG, int H, int W, int C, int ksize, int dtype_fp32, float* ws, void* dx,
+                               float* dw, void* stream);
+
 /* Pixel shuffle of ConvTranspose2d(k=2, stride=2) (unet.py:90) with the F.pad offsets of unet.py:95-97:
  * z [IMG][H][W][4][C] (+bias) <-> y [IMG][Hd][Wd][C] at (2h+i+oy, 2w+j+ox), tap = 2i+j. */
 int b200_shuffle2x2(const void* src, void* dst, const float* bias, long long IMG, int H, int W, int C, int Hd,

@@ -218,17 +218,21 @@ class OutConv(nn.Module):
 
 
 class SpatialAttention(nn.Module):
-    """Optional bottleneck attention (reference unet.py:113-125).  Every caller of the reference
-    passes use_attention=False, so this stays a plain PyTorch module outside the accelerated path."""
+    """Optional bottleneck attention (reference unet.py:113-125): x * sigmoid(conv_k([mean_c x ; amax_c x])), on the
+    kernels of csrc/attention.cu (kernel_size 1, 3, 5 or 7; any other size raises at the first call)."""
 
     def __init__(self, kernel_size=7):
         super().__init__()
         self.conv = nn.Conv2d(2, 1, kernel_size, padding=kernel_size // 2, bias=False)
         self.sigmoid = nn.Sigmoid()
 
+    def _seq(self, x):
+        """x [T,B,H,W,C] channels-last in the activation dtype -> the same shape and dtype."""
+        return Fn.SpatialAttention.apply(x, self.conv.weight)
+
     def forward(self, x):
-        pooled = torch.cat([x.mean(dim=1, keepdim=True), x.amax(dim=1, keepdim=True)], dim=1)
-        return x * self.sigmoid(self.conv(pooled))
+        _require_cuda(x, "SpatialAttention")
+        return _to_nchw(self._seq(_to_nhwc(x)))
 
 
 # -----------------------------------------------------------------------------------------------
@@ -267,9 +271,7 @@ class TemporalUNetDualView(nn.Module):
         x3, p3 = self.down3._seq_pooled(p2, True)
         xb = self.bottleneck._seq_pooled(p3)
         if self.use_attention:
-            T, B, H, W, C = xb.shape
-            a = self.attention(xb.reshape(T * B, H, W, C).permute(0, 3, 1, 2).float())
-            xb = a.permute(0, 2, 3, 1).reshape(T, B, H, W, C).to(xb.dtype).contiguous()
+            xb = self.attention._seq(xb)
         return xb, (x3, x2, x1, x0)
 
     def encode_once(self, x_t):

@@ -60,12 +60,16 @@ KERNELS_PER_CALL = {
     "b200_maxpool2_fwd": 1, "b200_maxpool2_bwd": 1, "b200_bn_relu_apply_pool": 1, "b200_bn_relu_pool_bwd_reduce": 1,
     "b200_bn_relu_pool_bwd_apply": 1, "b200_bn_relu_outconv_fwd": 1, "b200_bn_relu_outconv_bwd_reduce": 2,
     "b200_bn_relu_outconv_bwd_apply": 1, "b200_lstm_gates_fwd": 1, "b200_lstm_gates_bwd": 1,
-    "b200_colsum": 2, "b200_wl1_grad_loss_fwd": 2, "b200_wl1_grad_loss_bwd": 1, "b200_denorm_metrics_accum": 1, "b200_sequence_batch": 1, "b200_pack_weight": 1, "b200_unpack_wgrad": 1, "b200_grad_sqnorm_multi": 1, "b200_grad_clip_multi": 1, "b200_adamw_multi": 1, "b200_adamw_pack": 1, "b200_adamw_pack_multi": 1, "b200_outconv_fwd": 1, "b200_outconv_bwd": 5, "b200_shuffle2x2": 1, "b200_strided_copy": 1,
+    "b200_colsum": 2, "b200_wl1_grad_loss_fwd": 2, "b200_wl1_grad_loss_bwd": 1, "b200_denorm_metrics_accum": 1, "b200_sequence_batch": 1, "b200_pack_weight": 1, "b200_unpack_wgrad": 1, "b200_grad_sqnorm_multi": 1, "b200_grad_clip_multi": 1, "b200_adamw_multi": 1, "b200_adamw_pack": 1, "b200_adamw_pack_multi": 1, "b200_outconv_fwd": 1, "b200_outconv_bwd": 5, "b200_spatial_attention_fwd": 2, "b200_spatial_attention_bwd": 4, "b200_shuffle2x2": 1, "b200_strided_copy": 1,
 }
 
 
+# launches of calls whose count depends on their arguments (call(..., kernels=n)) beyond KERNELS_PER_CALL's figure
+_KERNELS_ADJUST = [0]
+
+
 def kernel_launches() -> int:
-    return sum(KERNELS_PER_CALL.get(k, 1) * v for k, v in CALLS.items())
+    return sum(KERNELS_PER_CALL.get(k, 1) * v for k, v in CALLS.items()) + _KERNELS_ADJUST[0]
 
 
 def lib():
@@ -129,8 +133,9 @@ def _is_tensor(a) -> bool:
     return hasattr(a, "data_ptr")
 
 
-def call(name: str, *args, tag: str = "", work=None):
-    """Calls an int-returning entry point and raises on a non-zero status.  Pointer arguments may be tensors (or None)."""
+def call(name: str, *args, tag: str = "", work=None, kernels=None):
+    """Calls an int-returning entry point and raises on a non-zero status.  Pointer arguments may be tensors (or None).
+    kernels: the number of kernels this call launches, where it depends on the arguments (else KERNELS_PER_CALL)."""
     timer = TIMER
     if timer is not None:
         import torch
@@ -153,6 +158,8 @@ def call(name: str, *args, tag: str = "", work=None):
         e1.record()
         timer.append((name + (" " + tag if tag else ""), e0, e1, work, torch.cuda.current_stream().cuda_stream))
     CALLS[name] = CALLS.get(name, 0) + 1
+    if kernels is not None:
+        _KERNELS_ADJUST[0] += kernels - KERNELS_PER_CALL.get(name, 1)
     if rc != 0:
         raise RuntimeError(f"{name} failed: rc={rc}: {last_error()}")
 

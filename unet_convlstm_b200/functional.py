@@ -553,3 +553,29 @@ class ConvLSTMSeq(torch.autograd.Function):
             bg.keep(dweight, dbias)
         ctx.h_all = ctx.c_all = ctx.gates = None
         return dx_seq, dh0, dc0, dweight, dbias, None
+
+
+# ------------------------------------------------------------------------------------------------
+# SpatialAttention (unet.py:113-125), the optional bottleneck attention of TemporalUNetDualView
+# ------------------------------------------------------------------------------------------------
+class SpatialAttention(torch.autograd.Function):
+    """y = x * a, a = sigmoid(conv_k([mean_c x ; amax_c x])) per image of x [T,B,H,W,C] (weight: the nn.Conv2d weight
+    [1, 2, k, k], read by the kernels as it is: no packed copy).  The pooled map and a (fp32, one or two values per
+    pixel) are kept for backward with x; the gradient of the max goes to every tied maximum in equal parts, as
+    torch.amax's does."""
+
+    @staticmethod
+    def forward(ctx, x, weight):
+        x = _c(x)
+        w = _c(weight.detach())
+        y, pooled, a = ops.spatial_attention_fwd(x, w)
+        ctx.save_for_backward(x, weight, pooled, a)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, weight, pooled, a = ctx.saved_tensors
+        dy = _c(dy)
+        dx, dw = ops.spatial_attention_bwd(x, dy if dy.dtype == x.dtype else dy.to(x.dtype), _c(weight.detach()), pooled,
+                                           a, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        return dx, dw

@@ -614,6 +614,52 @@ def outconv_bwd(x, w, dy, need_dx=True):
 
 
 # ------------------------------------------------------------------------------------------------
+# SpatialAttention (unet.py:113-125): y = x * sigmoid(conv_k([mean_c x ; amax_c x]))
+# ------------------------------------------------------------------------------------------------
+ATTENTION_KSIZES = (1, 3, 5, 7)
+_ATTN_WGRAD_PIXELS = 2048   # pixels per partial weight-gradient sum of b200_spatial_attention_bwd
+
+
+def _attn_ksize(w):
+    k = w.shape[-1]
+    if w.dim() != 4 or tuple(w.shape[:2]) != (1, 2) or w.shape[2] != k or k not in ATTENTION_KSIZES:
+        raise RuntimeError(f"spatial attention: weight {tuple(w.shape)} is not supported: the kernels take [1, 2, k, k] with "
+                           f"k in {ATTENTION_KSIZES} (there is no fallback)")
+    if w.dtype != torch.float32:
+        raise RuntimeError(f"spatial attention: weight dtype {w.dtype}, expected torch.float32")
+    return k
+
+
+def spatial_attention_fwd(x, w):
+    """x [T,B,H,W,C] (activation dtype), w fp32 [1,2,k,k] -> (y like x, pooled fp32 [T,B,H,W,2], a fp32 [T,B,H,W])."""
+    _chk(x, "x"), _chk(w, "w")
+    k = _attn_ksize(w)
+    T, B, H, W, C = x.shape
+    pooled = torch.empty((T, B, H, W, 2), device=x.device, dtype=torch.float32)
+    a = torch.empty((T, B, H, W), device=x.device, dtype=torch.float32)
+    y = torch.empty_like(x)
+    _lib.call("b200_spatial_attention_fwd", _p(x), _p(w), T * B, H, W, C, k, _f32(x), _p(pooled), _p(a), _p(y), _st(),
+              tag=f"C{C} {H}x{W} k{k}", work=(None, 3 * x.numel() * x.element_size()))   # x read twice, y written
+    return y, pooled, a
+
+
+def spatial_attention_bwd(x, dy, w, pooled, a, need_dx=True, need_dw=True):
+    """Returns (dx like x or None, dw fp32 [1,2,k,k] or None) for y = spatial_attention_fwd(x, w)[0] and dy = dL/dy."""
+    _chk(x, "x"), _chk(dy, "dy"), _chk(w, "w"), _chk(pooled, "pooled"), _chk(a, "a")
+    k = _attn_ksize(w)
+    T, B, H, W, C = x.shape
+    P = T * B * H * W
+    ws = torch.empty(2 * P + -(-P // _ATTN_WGRAD_PIXELS) * 2 * k * k, device=x.device, dtype=torch.float32)
+    dx = torch.empty_like(x) if need_dx else None
+    dw = torch.empty((1, 2, k, k), device=x.device, dtype=torch.float32) if need_dw else None
+    _lib.call("b200_spatial_attention_bwd", _p(x), _p(dy), _p(w), _p(pooled), _p(a), T * B, H, W, C, k, _f32(x), _p(ws),
+              _p(dx), _p(dw), _st(), tag=f"C{C} {H}x{W} k{k}",
+              work=(None, (2 + 3 * need_dx) * x.numel() * x.element_size()),   # (x, dy) read once or twice, dx written
+              kernels=2 + int(need_dx) + 2 * int(need_dw))
+    return dx, dw
+
+
+# ------------------------------------------------------------------------------------------------
 # ConvLSTM cell
 # ------------------------------------------------------------------------------------------------
 def lstm_tc_ok(x_t, Ch) -> bool:
